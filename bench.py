@@ -1,8 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the SpMV hot path (see BASELINE.json / BASELINE.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+Every timed SpMV loop runs exactly K steps (PageRank runs --pr-iters iterations).
+--dump-outputs DIR writes, after the timed steps, what each timed path computed in
+its last step as DIR/<name>.npy (float32, rank 0): every SpMV kernel, plan and
+host-buffer call timed on configs 2, 3 and 4, and every PageRank vector timed
+(one per graph: the transports are checked bit-identical).  Each file is the same
+seeded sample of DUMP_ROWS entries of its vector, so that two builds can be
+compared output for output on identical inputs.  The reference arm writes its
+config-2 y under the same name and sample (the positions inside its band).
 
 A "step" is one pass of the hot path over one batch of synthetic input: one
 ELL SpMV over BASELINE config 2 (5-point Laplacian on a 4096^2 grid, 16.7 M
@@ -50,6 +59,24 @@ sys.path.insert(0, ROOT)
 GRID = 4096            # BASELINE config 2
 SEED_X = 42
 FALLBACK_PEAK_GBS = 6650.0
+DUMP_ROWS = 1 << 19    # --dump-outputs: entries kept per output vector (15 vectors at most: 30 MiB)
+DUMP_SEED = 2024
+
+
+def dump_index(n):
+    """The sorted positions of an n-vector that --dump-outputs keeps: all of them, or a fixed seeded sample."""
+    import numpy as np
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+
+
+def write_outputs(directory, outputs):
+    """--dump-outputs: each float32 array of `outputs` as <directory>/<name>.npy."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def measured_peak():
@@ -178,7 +205,10 @@ def run_reference_arm(args):
     bytes_step = 8 * n * 5 + 4 * (n_full if n == n_full else n + GRID) + 4 * n
     for _ in range(max(args.warmup, 1) - 1):
         cpu_reference_time(rp, ci, va, x, n, n_full, 1)
-    sec, kind, threads, _ = cpu_reference_time(rp, ci, va, x, n, n_full, args.steps)
+    sec, kind, threads, y = cpu_reference_time(rp, ci, va, x, n, n_full, args.steps)
+    if args.dump_outputs is not None:
+        idx = dump_index(n_full)  # the GPU arm's sample of config-2 y; a band keeps the positions inside it
+        write_outputs(args.dump_outputs, {"config2_ell_y": y[idx[idx < n]]})
     gbs = bytes_step / sec / 1e9
     sample = ("the full config-2 matrix" if n == n_full else f"the first {n} rows (a band) of the config-2 matrix")
     line = {
@@ -346,6 +376,14 @@ def run_product_arm(args):
     def r4(v):
         return float(f"{v:.5g}")
 
+    outputs = {}
+
+    def keep_output(name, v):
+        """--dump-outputs: the sample of vector v (device or host) that is written as <name>.npy at the end."""
+        if args.dump_outputs is not None and rank == 0:
+            idx = torch.from_numpy(dump_index(v.numel())).to(v.device)
+            outputs[name] = v[idx].cpu().numpy().astype(np.float32)
+
     # ---- headline: config 2, ELL, one 16.7 M-row band per rank (weak scaling) -----------------
     log("config 2: build + ELL headline")
     n_loc = GRID * GRID
@@ -375,14 +413,18 @@ def run_product_arm(args):
     launches_before = sp.launch_count()
     ms = timed_region(torch, stream, ell_step, args.steps, dist_on)
     gpu_launches = sp.launch_count() - launches_before
-    # keep the GPU under the same load a little longer so the clock sampler sees it
-    if args.steps * (ms / args.steps) < 400:
-        timed_region(torch, stream, ell_step, int(400 / max(ms / args.steps, 1e-3)) + 1, dist_on)
+    y_device_path = y.clone()
+    torch.cuda.synchronize()  # the clone runs on the default stream, the load phase below rewrites y on `stream`
+    keep_output("config2_ell_y", y_device_path)
+    # untimed: keep the GPU under the same load for ~400 ms so the clock sampler sees it loaded
+    if ms < 400:
+        for _ in range(int(400 / max(ms / args.steps, 1e-3)) + 1):
+            ell_step()
+        torch.cuda.synchronize()
     clocks = sampler.stop()
     ms_per_step = ms / args.steps
     value = world * ell_bytes / (ms_per_step * 1e-3) / 1e9
     launch_gbs = ell_bytes / (ms_per_step * 1e-3) / 1e9
-    y_device_path = y.clone()
 
     # ---- e2e: the C-ABI call that takes HOST x / y (pinned); H2D, kernel, D2H inside the timed region ---
     log("e2e")
@@ -421,11 +463,12 @@ def run_product_arm(args):
         torch.cuda.synchronize()
         return max_over_ranks((time.perf_counter() - t0) / steps)
 
-    e2e_steps = max(3, min(args.steps, 10))
     y_host.zero_()
-    e2e_sec = wall_time(e2e_step, e2e_steps)
+    e2e_sec = wall_time(e2e_step, args.steps)
     e2e_same = bool(torch.equal(y_host.view(torch.int32), y_device_path.cpu().view(torch.int32)))
-    serial_sec = wall_time(e2e_serial_step, e2e_steps)
+    keep_output("config2_ell_host_y", y_host)
+    serial_sec = wall_time(e2e_serial_step, args.steps)
+    keep_output("config2_ell_host_serial_y", y_host)
     # still gated after the timed calls (a call whose x did not arrive in time would have fallen back for good)
     assert sp.lib.spmv_b200_ell_host_plan_gated(host_plan, C.byref(c_gated), None) == 0
     host_gated = bool(c_gated.value)
@@ -463,6 +506,7 @@ def run_product_arm(args):
                 A.ptr, sp.dptr(x), sp.dptr(y), C.byref(cfg), C.c_void_p(s_ptr)), csr_bytes, args.steps, args.warmup,
                 dist_on, world)
             torch.cuda.synchronize()
+            keep_output(f"config2_{name}_y", y)
             entry = {"gbs": r4(r["gbs"]), "ms": r4(r["ms_per_step"]), "frac": r4(r["gbs"] / world / peak),
                      "frac_of_8000": r4(r["gbs"] / world / 8000.0)}
             if kernel != sp.MERGE_PATH:  # sequential order: bit-identical to the ELL result (= spmv_cpu_*)
@@ -475,12 +519,14 @@ def run_product_arm(args):
         # segmented-stream kernel (csr_seg_kernels.cu)
         plan2 = sp.CsrPlan(A.ptr)
         r = bench_kernel(torch, sp, stream, lambda: plan2.spmv(x, y, s_ptr), csr_bytes, args.steps, args.warmup, dist_on, world)
+        keep_output("config2_csr_planned_y", y)
         extra["config2_csr_planned"] = {"gbs": r4(r["gbs"]), "ms": r4(r["ms_per_step"]), "frac": r4(r["gbs"] / world / peak),
                                         "plan_mode": plan2.info()[2]}
         plan2.close()
         # and with the caller's permission to snapshot the values: the plan re-lays the matrix out as ELL
         plan3 = sp.CsrPlan(A.ptr, snapshot_values=True)
         r = bench_kernel(torch, sp, stream, lambda: plan3.spmv(x, y, s_ptr), csr_bytes, args.steps, args.warmup, dist_on, world)
+        keep_output("config2_csr_planned_value_snapshot_y", y)
         extra["config2_csr_planned_value_snapshot"] = {
             "gbs": r4(r["gbs"]), "ms": r4(r["ms_per_step"]), "frac": r4(r["gbs"] / world / peak), "plan_mode": plan3.info()[2],
             "note": "CSR algorithmic bytes over the time of the ELL kernel the plan routes to (it moves 805 MB)"}
@@ -501,9 +547,10 @@ def run_product_arm(args):
         for kernel, name in ((sp.SCALAR_CSR, "csr_scalar"), (sp.MERGE_PATH, "csr_merge")):
             cfg = sp.make_config(kernel)
             r = bench_kernel(torch, sp, stream, lambda: sp.lib.spmv_b200_spmv_csr_async(
-                A3.ptr, sp.dptr(x3), sp.dptr(y3), C.byref(cfg), C.c_void_p(s_ptr)), b3, max(5, args.steps // 2), 3)
+                A3.ptr, sp.dptr(x3), sp.dptr(y3), C.byref(cfg), C.c_void_p(s_ptr)), b3, args.steps, 3)
             extra[f"config3_{name}"] = {"gbs": r4(r["gbs"]), "ms": r4(r["ms_per_step"]), "frac": r4(r["gbs"] / peak),
                                         "rows": rows3, "nnz": ci3.numel()}
+            keep_output(f"config3_{name}_y", y3)
         extra["config3_selector"] = "MERGE_PATH (outlier override; reference policy: SCALAR_CSR)"
         scalars["config3_merge_frac"] = extra["config3_csr_merge"]["frac"]
         del A3, rp3, ci3, va3, x3, y3
@@ -526,12 +573,13 @@ def run_product_arm(args):
         cfg = sp.make_config(sp.MERGE_PATH)
         log(f"R-MAT scale {scale}: csr_merge")
         r = bench_kernel(torch, sp, stream, lambda: sp.lib.spmv_b200_spmv_csr_async(
-            csr.ptr, sp.dptr(xg), sp.dptr(y_slice), C.byref(cfg), C.c_void_p(s_ptr)), 0, max(5, args.steps // 2), 3, dist_on)
+            csr.ptr, sp.dptr(xg), sp.dptr(y_slice), C.byref(cfg), C.c_void_p(s_ptr)), 0, args.steps, 3, dist_on)
         gbs = tot / (r["ms_per_step"] * 1e-3) / 1e9
         extra[f"rmat{scale}_csr_merge"] = {"gbs": r4(gbs), "ms": r4(r["ms_per_step"]), "frac": r4(gbs / world / peak),
                                            "nnz": n_edges, "rows": n, "scaling": "strong (one graph, row shards)"}
         torch.cuda.synchronize()
         y_ref = y_slice.clone()
+        keep_output(f"rmat{scale}_csr_merge_y", y_ref[:rows_p])
         # the same product through a CSR plan: merge coordinates computed once + hub-column table
         # (csr_hot_kernels.cu) for scale-free shards; bit-identical results, checked here on the full-size shard
         log(f"R-MAT scale {scale}: csr_merge through a CSR plan")
@@ -540,8 +588,9 @@ def run_product_arm(args):
         torch.cuda.synchronize()
         plan_ms = (time.perf_counter() - t0) * 1e3
         hot_columns, hot_nnz, hot_mode = plan.info()
-        r = bench_kernel(torch, sp, stream, lambda: plan.spmv(xg, y_slice, s_ptr), 0, max(5, args.steps // 2), 3, dist_on)
+        r = bench_kernel(torch, sp, stream, lambda: plan.spmv(xg, y_slice, s_ptr), 0, args.steps, 3, dist_on)
         torch.cuda.synchronize()
+        keep_output(f"rmat{scale}_csr_merge_plan_y", y_slice[:rows_p])
         same = all_ok(bool(torch.equal(y_ref.view(torch.int32), y_slice.view(torch.int32))))
         gbs = tot / (r["ms_per_step"] * 1e-3) / 1e9
         extra[f"rmat{scale}_csr_merge_plan"] = {
@@ -629,6 +678,8 @@ def run_product_arm(args):
                 sec = t if sec is None else min(sec, t)
             link1 = nvlink_bytes(local_rank) if link0 is not None else None
             vec = pr.ranks(dev)
+            if mode == modes[0]:  # the transports are checked bit-identical below
+                keep_output(f"pagerank{tag}_ranks", vec)
             total = float(vec.double().sum().item())
             checks[mode] = vector_checksum(torch, vec) + (total,)
             entry = {"iters_per_s": r4(iters / sec), "ms_per_iter": r4(sec / iters * 1e3), "exchange": used,
@@ -687,6 +738,7 @@ def run_product_arm(args):
             for _ in range(2):
                 res = pr.run(0.85, 0.0, 0, fixed_iterations=args.pr_iters)
                 sec = res.device_seconds if sec == 0.0 else min(sec, res.device_seconds)
+            keep_output("pagerank_1gpu_ranks", pr.ranks(dev))
             pr.close()
             c1.close()
             del csr, srp, sci, sva
@@ -742,6 +794,8 @@ def run_product_arm(args):
         }
         line.update(scalars)
         line["extra"] = extra
+        if args.dump_outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         sys.stdout.flush()
         os.dup2(real_stdout, 1)
         print(json.dumps(line), flush=True)
@@ -777,7 +831,12 @@ def main():
     ap.add_argument("--pr-one-gpu", type=int, default=1,
                     help="N > 1: rank 0 also runs the whole PageRank graph on its GPU alone (pagerank_1gpu_iters_per_s, "
                          "pagerank_speedup_vs_1gpu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed seeded sample of every timed path's output after its last step as DIR/<name>.npy "
+                         "(float32, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
