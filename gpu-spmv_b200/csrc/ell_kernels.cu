@@ -344,9 +344,17 @@ cudaError_t launch_tma_pipe(int rows, int width, const int* ci, const float* va,
     // thread slot of the SM, the ring only needs two stages -> 2 stages, as many CTAs as fit (<= 8).
     int stages = env_stages > 0 ? env_stages : 2;
     if (stages > 16) stages = 16;
+    // a deeper ring than one CTA's shared memory holds is cut to what fits (W = 8, one row per thread:
+    // 16 KiB per stage, so 16 stages would ask for 256 KiB)
+    int dev_id = 0, optin = 0;
+    cudaGetDevice(&dev_id);
+    cudaError_t e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev_id);
+    if (e != cudaSuccess) return e;
+    const int fit_stages = static_cast<int>((static_cast<size_t>(optin) - 128) / stage_bytes);
+    if (stages > fit_stages) stages = fit_stages;
     if (stages < 2) stages = 2;
     const size_t smem = 128 + stages * stage_bytes;
-    cudaError_t e = cudaFuncSetAttribute(ell_tma_pipe_kernel<RPT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    e = cudaFuncSetAttribute(ell_tma_pipe_kernel<RPT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     // a persistent grid must not exceed what is co-resident (registers and shared memory)
@@ -355,8 +363,7 @@ cudaError_t launch_tma_pipe(int rows, int width, const int* ci, const float* va,
     if (e != cudaSuccess) return e;
     if (fit < 1) fit = 1;
     const int ctas_per_sm = (env_ctas > 0 && env_ctas < fit) ? env_ctas : fit;
-    int sms = 148, dev_id = 0;
-    cudaGetDevice(&dev_id);
+    int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev_id);
     const int num_windows = static_cast<int>((static_cast<long long>(row_hi - row_lo) + kWindow - 1) / kWindow);
     if (num_windows <= 0) return cudaSuccess;

@@ -7,6 +7,22 @@ def bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
 
 
+def bits_nan_as_class(a):
+    """bits() with every NaN written as 0x7FC00000.  The sign and payload of a NaN are not part of the
+    result: x86 keeps an input NaN's payload and gives 0xFFC00000 for 0 * Inf, the GPU gives 0x7FFFFFFF."""
+    b = bits(a).copy()
+    b[np.isnan(np.asarray(a, dtype=np.float32))] = 0x7FC00000
+    return b
+
+
+def assert_same_bits_nan_as_class(y, ref, what=""):
+    """Bit-identical results, every NaN counted as one value."""
+    by, br = bits_nan_as_class(y), bits_nan_as_class(ref)
+    bad = np.flatnonzero(by != br)
+    assert bad.size == 0, (f"{what}: {bad.size} rows differ in their bits, first row {bad[0]}: "
+                           f"{y[bad[0]]!r} (0x{by[bad[0]]:08x}) against {ref[bad[0]]!r} (0x{br[bad[0]]:08x})")
+
+
 class GpuCSR:
     """Library-owned CSR (host arrays + csr_to_gpu), freed on close()."""
 
