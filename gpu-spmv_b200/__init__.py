@@ -399,6 +399,47 @@ def pagerank_device_history(adj_matrix, d_ranks, config=None, capacity=100):
     return rc, it.value, res.value, conv.value, hist
 
 
+def _personalization(personalization, n):
+    """Host float32 copy of a personalization vector of n entries, or None."""
+    if personalization is None:
+        return None
+    v = np.ascontiguousarray(personalization, dtype=np.float32)
+    if v.ndim != 1 or v.size != n:
+        raise ValueError(f"personalization must hold {n} entries, got shape {v.shape}")
+    return v
+
+
+def pagerank_personalized(adj_matrix, personalization, config=None):
+    """Personalized PageRank: teleport and dangling mass follow `personalization` (non-negative host
+    array of num_rows entries, normalised by the library; None: pagerank()).  Returns
+    (PageRankResult, ranks ndarray copy); call pagerank_free(result) when done.  Raises on a rejected
+    vector (NaN, Inf, negative entry, zero sum)."""
+    n = adj_matrix.contents.num_rows if adj_matrix else 0
+    v = _personalization(personalization, n)
+    res = PageRankResult()
+    cfg = C.byref(config) if config is not None else None
+    rc = lib.spmv_b200_pagerank_personalized(adj_matrix, cfg, v.ctypes.data_as(capi.c_float_p) if v is not None else None,
+                                             C.byref(res))
+    if rc != 0:
+        raise RuntimeError(f"pagerank_personalized: {spmv_error_string(rc)}")
+    ranks = host_array(res.ranks, n, np.float32).copy() if res.ranks else None
+    return res, ranks
+
+
+def pagerank_device_personalized(adj_matrix, d_ranks, personalization, config=None, capacity=0):
+    """pagerank_device for personalized PageRank (see pagerank_personalized); d_ranks (torch float32 [n])
+    receives the ranks -> (rc, iterations, residual, converged, l1, history of `capacity` L2 residuals)."""
+    n = adj_matrix.contents.num_rows if adj_matrix else 0
+    v = _personalization(personalization, n)
+    it, res, conv, l1 = C.c_int(0), C.c_float(0), C.c_bool(False), C.c_double(0)
+    hist = np.full(capacity, np.nan, dtype=np.float32)
+    cfg = C.byref(config) if config is not None else None
+    rc = lib.spmv_b200_pagerank_device_personalized(
+        adj_matrix, cfg, v.ctypes.data_as(capi.c_float_p) if v is not None else None, dptr(d_ranks), C.byref(it),
+        C.byref(res), C.byref(conv), C.byref(l1), hist.ctypes.data_as(capi.c_float_p) if capacity > 0 else None, capacity)
+    return rc, it.value, res.value, conv.value, l1.value, hist
+
+
 # --------------------------------------------------------------- benchmark ----
 
 def make_bench_config(num_warmup_runs=5, num_runs=20, compare_cpu=True):

@@ -200,6 +200,12 @@ PROTOTYPES = {
     "spmv_b200_pagerank_device_history": (C.c_int, [CSR_P, PRC_P, vp, c_int_p, c_float_p, C.POINTER(C.c_bool), c_float_p,
                                            C.c_int]),
     "spmv_b200_pagerank_device": (C.c_int, [CSR_P, PRC_P, vp, c_int_p, c_float_p, C.POINTER(C.c_bool), c_double_p]),
+    "spmv_b200_pagerank_personalized": (C.c_int, [CSR_P, PRC_P, c_float_p, PRR_P]),
+    "spmv_b200_pagerank_device_personalized": (C.c_int, [CSR_P, PRC_P, c_float_p, vp, c_int_p, c_float_p,
+                                                         C.POINTER(C.c_bool), c_double_p, c_float_p, C.c_int]),
+    "spmv_b200_pagerank_multi_personalized": (C.c_int, [CSR_P, vp, c_float_p, C.c_int, c_int_p, C.c_int, C.c_int, C.c_int,
+                                                        vp, vp]),
+    "spmv_b200_pr_dist_set_personalization": (C.c_int, [vp, c_float_p]),
 }
 
 

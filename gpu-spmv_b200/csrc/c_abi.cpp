@@ -254,6 +254,19 @@ int spmv_b200_pagerank(const spmv_b200_csr* adj, const spmv_b200_pagerank_config
         return 0;
     });
 }
+int spmv_b200_pagerank_personalized(const spmv_b200_csr* adj, const spmv_b200_pagerank_config* config,
+                                    const float* personalization, spmv_b200_pagerank_result* out) {
+    if (!adj || !out) return kBadArg;
+    return guarded([&] {
+        PageRankResult r;
+        const int rc = b200::pagerank_to_host(cpp(adj), cpp(config), personalization, &r);
+        out->ranks = r.ranks;
+        out->iterations = r.iterations;
+        out->final_residual = r.final_residual;
+        out->converged = r.converged;
+        return rc;
+    });
+}
 void spmv_b200_pagerank_free(spmv_b200_pagerank_result* r) { pagerank_free(reinterpret_cast<PageRankResult*>(r)); }
 int spmv_b200_pagerank_top_k(const spmv_b200_pagerank_result* r, int num_nodes, int k, spmv_b200_topk_node* top_k) {
     if (!r || !r->ranks || !top_k || k <= 0) return kBadArg;
@@ -658,6 +671,23 @@ int spmv_b200_pagerank_device(const spmv_b200_csr* adj, const spmv_b200_pagerank
     });
 }
 
+int spmv_b200_pagerank_device_personalized(const spmv_b200_csr* adj, const spmv_b200_pagerank_config* config,
+                                           const float* personalization, float* d_ranks, int* iterations,
+                                           float* final_residual, bool* converged, double* l1_residual,
+                                           float* l2_history, int history_capacity) {
+    if (!adj || !d_ranks || history_capacity < 0 || (history_capacity > 0 && !l2_history)) return kBadArg;
+    return guarded([&] {
+        float* d_pvec = nullptr;
+        int rc = b200::pr_personalization_upload(personalization, cpp(adj)->num_rows, 0, cpp(adj)->num_rows, &d_pvec,
+                                                  nullptr);
+        if (rc != 0) return rc;
+        rc = b200::pagerank_device(cpp(adj), cpp(config), d_ranks, iterations, final_residual, converged, l1_residual, true,
+                                   l2_history, history_capacity, d_pvec);
+        cudaFree(d_pvec);
+        return rc;
+    });
+}
+
 }  // extern "C"
 
 // ---- multi-GPU PageRank ---------------------------------------------------------------------
@@ -672,6 +702,15 @@ int spmv_b200_pagerank_multi(const spmv_b200_csr* adj, const spmv_b200_pagerank_
     return guarded([&] {
         return b200::pagerank_multi(cpp(adj), cpp(config), n_gpus, devices, exchange, row_weight, fixed_iterations,
                                     ranks_out, reinterpret_cast<b200::PrDistResult*>(out));
+    });
+}
+int spmv_b200_pagerank_multi_personalized(const spmv_b200_csr* adj, const spmv_b200_pagerank_config* config,
+                                          const float* personalization, int n_gpus, const int* devices, int exchange,
+                                          int row_weight, int fixed_iterations, float* ranks_out,
+                                          spmv_b200_pr_dist_result* out) {
+    return guarded([&] {
+        return b200::pagerank_multi(cpp(adj), cpp(config), n_gpus, devices, exchange, row_weight, fixed_iterations,
+                                    ranks_out, reinterpret_cast<b200::PrDistResult*>(out), personalization);
     });
 }
 int spmv_b200_comm_create(int rank, int world, const char* session, int timeout_s, spmv_b200_comm** out) {
@@ -707,6 +746,9 @@ int spmv_b200_pr_dist_run(spmv_b200_pr_dist* d, const spmv_b200_pagerank_config*
         return b200::pr_dist_run(reinterpret_cast<b200::PrDist*>(d), cpp(config), fixed_iterations,
                                  reinterpret_cast<b200::PrDistResult*>(out));
     });
+}
+int spmv_b200_pr_dist_set_personalization(spmv_b200_pr_dist* d, const float* personalization) {
+    return guarded([&] { return b200::pr_dist_set_personalization(reinterpret_cast<b200::PrDist*>(d), personalization); });
 }
 const float* spmv_b200_pr_dist_ranks(const spmv_b200_pr_dist* d) { return b200::pr_dist_ranks(reinterpret_cast<const b200::PrDist*>(d)); }
 int spmv_b200_pr_dist_exchange(const spmv_b200_pr_dist* d) { return b200::pr_dist_exchange(reinterpret_cast<const b200::PrDist*>(d)); }

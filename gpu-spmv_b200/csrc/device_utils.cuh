@@ -144,6 +144,29 @@ __device__ __forceinline__ bool aligned16(const void* p) {
     return (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
 }
 
+// ---- PageRank row update ------------------------------------------------------
+// The one definition of the update, used by every PageRank epilogue (PageRankRowT::finish and
+// ::tile_epilogue, seg_pagerank_epilogue_kernel, pagerank_small_kernel).  pvec selects the form
+// at run time; the branch is uniform over the kernel.
+//   pvec == nullptr  global PageRank:      r = (d*y + d*D/n) + teleport,          teleport = (1-d)/n
+//   pvec != nullptr  personalized PageRank: r = (d*y + (d*D)*v[i]) + teleport*v[i], teleport = 1-d
+// D is the dangling mass of r_old and v the normalised personalization vector.  Every operation
+// is rounded separately (no FMA contraction), so the global form is exactly the reference's
+// expression (src/pagerank.cu:111-113, left to right in fp32).
+// Per-step context: d*D/n, or d*D in the personalized form.
+__device__ __forceinline__ float pr_step_context(float damping, float dsum, int n, const float* pvec) {
+    const float dd = __fmul_rn(damping, dsum);
+    return pvec ? dd : __fdiv_rn(dd, static_cast<float>(n));
+}
+// New rank of one row from its product y; local_row indexes pvec (the rows of this shard).
+__device__ __forceinline__ float pr_row_value(float damping, float y, float ctx, float teleport, const float* pvec,
+                                              int local_row) {
+    const float dy = __fmul_rn(damping, y);
+    if (!pvec) return __fadd_rn(__fadd_rn(dy, ctx), teleport);
+    const float v = __ldg(pvec + local_row);
+    return __fadd_rn(__fadd_rn(dy, __fmul_rn(ctx, v)), __fmul_rn(teleport, v));
+}
+
 // ---- warp reductions ---------------------------------------------------------
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -7,6 +7,7 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <vector>
 
 namespace spmv {
 namespace b200 {
@@ -111,7 +112,7 @@ struct PageRankStepArgs {
     int row_offset;         // first global row of this shard
     int n_global;
     float damping;
-    float teleport;         // (1 - d) / n, computed on the host in fp32
+    float teleport;         // (1 - d) / n, or 1 - d when pvec is set; computed on the host in fp32
     const float* d_dsum;    // device scalar: dangling mass of r_old
     const uint32_t* bits;   // dangling bitmask over global node ids
     double* out;            // device [3]: sum d^2, sum |d|, next dangling mass
@@ -125,6 +126,10 @@ struct PageRankStepArgs {
     // r_new buffer of every GPU of the group (this one included) instead of n_peers - 1 unicast
     // stores, so the NVLink egress of a rank is 4 bytes per owned row instead of 4 * (n_peers - 1).
     float* mc_r_new;
+    // personalized PageRank: the normalised personalization vector (sums to 1) over the rows OF
+    // THIS SHARD, indexed by local row (global row - row_offset).  Teleport and dangling mass are
+    // spread by it instead of uniformly (dev::pr_row_value).  nullptr: global PageRank.
+    const float* pvec;
 };
 
 // ---- kernel launchers (stream-ordered; return the launch status) --------------------
@@ -304,14 +309,30 @@ struct PrPlan;
 int pr_plan_create(const CSRMatrix* shard, int row_offset, int n_global, cudaStream_t stream, PrPlan** out);
 void pr_plan_destroy(PrPlan* plan);
 int pr_plan_set_hot(PrPlan* plan, int max_hot_columns, bool force, cudaStream_t stream);
+// d_pvec: this shard's rows of the normalised personalization vector (PageRankStepArgs::pvec), or nullptr
 int pr_step(PrPlan* plan, const float* d_r_old, float* d_r_new, float damping, const float* d_dsum,
             const uint32_t* d_bits, double* d_partial, cudaStream_t stream,
-            float* const* peer_r_new = nullptr, int n_peers = 0, int self_rank = 0, float* mc_r_new = nullptr);
+            float* const* peer_r_new = nullptr, int n_peers = 0, int self_rank = 0, float* mc_r_new = nullptr,
+            const float* d_pvec = nullptr);
 const CsrView& pr_plan_view(const PrPlan* plan);
 int pr_plan_hub_columns(const PrPlan* plan);  // entries of the shared-memory x table in use (0: none)
 double* pr_plan_tmp(PrPlan* plan);
+// d_pvec: the normalised personalization vector [n] on the device (pr_personalization_upload), or nullptr
 int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d_ranks, int* iterations,
-                    float* final_residual, bool* converged, double* l1_residual, bool normalize = true, float* l2_history = nullptr, int history_capacity = 0);
+                    float* final_residual, bool* converged, double* l1_residual, bool normalize = true, float* l2_history = nullptr, int history_capacity = 0,
+                    const float* d_pvec = nullptr);
+// pagerank()'s body: host ranks in *result (new[]; nullptr on a failed validation).  personalization: host [n]
+// or nullptr (global PageRank, exactly pagerank()).  Returns INVALID_ARGUMENT for a rejected personalization.
+int pagerank_to_host(const CSRMatrix* adj, const PageRankConfig* config, const float* personalization,
+                     PageRankResult* result);
+// Personalization vector v (host, n entries): rejected (INVALID_ARGUMENT) when an entry is NaN, +-Inf or
+// negative, or when the f64 sum of the entries, in index order, is 0.  vhat[i] = (float)((double)v[i] / sum).
+// Host code only: every rank of a sharded run computes the same vhat from the same v.
+int pr_personalization_normalise(const float* v, int n, std::vector<float>* vhat);
+// Validates and normalises v as above, then copies rows [row_lo, row_lo + rows) of vhat into a new device
+// buffer of max(rows, 1) floats (*d_out; cudaFree it), complete on return (`stream` is synchronised).
+// v == nullptr: *d_out = nullptr, success.
+int pr_personalization_upload(const float* v, int n, int row_lo, int rows, float** d_out, cudaStream_t stream);
 
 }  // namespace b200
 }  // namespace spmv

@@ -232,6 +232,7 @@ struct PrDist {
     double* d_partial = nullptr;   // this rank's {sum d^2, sum |d|, dangling}
     double* d_gathered = nullptr;  // NCCL mode: world x 3
     float* d_out = nullptr;        // normalised result (full length)
+    float* d_pvec = nullptr;       // this shard's rows of the normalised personalization vector, or nullptr
     HostHistoryEntry* hist = nullptr;  // mapped pinned
     HostHistoryEntry* d_hist = nullptr;
     int hist_cap = 0;
@@ -258,7 +259,7 @@ void free_all(PrDist* d) {
     }
     cudaFree(d->plain_r[0]); cudaFree(d->plain_r[1]);
     cudaFree(d->d_state); cudaFree(d->d_bits); cudaFree(d->d_dsum); cudaFree(d->d_partial);
-    cudaFree(d->d_gathered); cudaFree(d->d_out);
+    cudaFree(d->d_gathered); cudaFree(d->d_out); cudaFree(d->d_pvec);
     if (d->hist) cudaFreeHost(d->hist);
     if (d->stream) cudaStreamDestroy(d->stream);
     delete d;
@@ -375,6 +376,31 @@ void pr_dist_destroy(PrDist* d) {
     free_all(d);
 }
 
+int pr_dist_set_personalization(PrDist* d, const float* v_host) {
+    if (!d) return static_cast<int>(SpMVError::INVALID_ARGUMENT);
+    if (v_host) {  // the same host code on every rank: a vector one rank rejects, every rank rejects
+        std::vector<float> vhat;
+        const int rc = pr_personalization_normalise(v_host, d->n, &vhat);
+        if (rc != 0) return rc;
+    }
+    // nothing of an earlier run still reads the old slice, and the cached iteration graphs, which hold its
+    // address (or none), are dropped: the next run captures them again
+    cudaStreamSynchronize(d->stream);
+    for (int q = 0; q < 2; ++q) {
+        if (d->graph[q]) cudaGraphExecDestroy(d->graph[q]);
+        d->graph[q] = nullptr;
+    }
+    cudaFree(d->d_pvec);
+    d->d_pvec = nullptr;
+    int rc = pr_personalization_upload(v_host, d->n, d->row_offset, d->rows, &d->d_pvec, d->stream);
+    if (!agree(d->comm, rc == 0)) {  // every rank runs the same form, or none keeps a vector
+        cudaFree(d->d_pvec);
+        d->d_pvec = nullptr;
+        if (rc == 0) rc = static_cast<int>(SpMVError::CUDA_MALLOC);
+    }
+    return rc;
+}
+
 int pr_dist_exchange(const PrDist* d) { return d ? d->exchange : -1; }
 const float* pr_dist_ranks(const PrDist* d) { return d ? d->d_out : nullptr; }
 cudaStream_t pr_dist_stream(const PrDist* d) { return d ? d->stream : nullptr; }
@@ -468,7 +494,7 @@ int enqueue_iteration(PrDist* d, int from, float damping) {
         if (d->exchange == kExchangeMulticast) mc = static_cast<float*>(d->r[to].mc);
     }
     int rc = pr_step(d->plan, d->vec(from), d->vec(to), damping, d->d_dsum, d->d_bits, d->d_partial, d->stream,
-                     fused ? peers : nullptr, fused ? d->world : 0, d->rank, mc);
+                     fused ? peers : nullptr, fused ? d->world : 0, d->rank, mc, d->d_pvec);
     if (rc != 0) return rc;
     if (fused) {
         PeerControl pc;

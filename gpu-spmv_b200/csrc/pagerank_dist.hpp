@@ -37,6 +37,10 @@ int pr_dist_create(Comm* comm, const CSRMatrix* shard, int row_offset, int n_glo
 void pr_dist_destroy(PrDist* d);  // collective
 // collective; fixed_iterations > 0 runs exactly that many iterations (no stop rule)
 int pr_dist_run(PrDist* d, const PageRankConfig* config, int fixed_iterations, PrDistResult* out);
+// collective; personalized PageRank from the next run on: v_host is the FULL host vector (n_global entries, the
+// same on every rank), validated and normalised as pr_personalization_normalise does; this rank keeps its rows.
+// nullptr returns to global PageRank.  Drops the cached iteration graphs.
+int pr_dist_set_personalization(PrDist* d, const float* v_host);
 int pr_dist_exchange(const PrDist* d);
 const float* pr_dist_ranks(const PrDist* d);  // device, full length, normalised; valid after a run
 cudaStream_t pr_dist_stream(const PrDist* d);
@@ -44,8 +48,10 @@ int pr_dist_hub_columns(const PrDist* d);
 
 // One process, n_gpus devices: adj is a HOST CSR; cuts nnz-balanced row shards (work(row) = nnz +
 // row_weight), uploads one per device and runs the loop with one host thread per device.
+// personalization: host [num_rows] or nullptr (pr_dist_set_personalization).
 int pagerank_multi(const CSRMatrix* adj, const PageRankConfig* config, int n_gpus, const int* devices, int exchange,
-                   int row_weight, int fixed_iterations, float* ranks_out, PrDistResult* out);
+                   int row_weight, int fixed_iterations, float* ranks_out, PrDistResult* out,
+                   const float* personalization = nullptr);
 
 }  // namespace b200
 }  // namespace spmv

@@ -18,8 +18,14 @@ namespace spmv {
 namespace b200 {
 
 int pagerank_multi(const CSRMatrix* adj, const PageRankConfig* config, int n_gpus, const int* devices, int exchange,
-                   int row_weight, int fixed_iterations, float* ranks_out, PrDistResult* out) {
+                   int row_weight, int fixed_iterations, float* ranks_out, PrDistResult* out,
+                   const float* personalization) {
     if (!adj || !ranks_out || n_gpus < 1 || n_gpus > 8) return static_cast<int>(SpMVError::INVALID_ARGUMENT);
+    if (personalization) {  // rejected before any device work (every rank checks it again)
+        std::vector<float> vhat;
+        const int rc = pr_personalization_normalise(personalization, adj->num_rows, &vhat);
+        if (rc != 0) return rc;
+    }
     if (!adj->row_ptrs || (adj->nnz > 0 && (!adj->col_indices || !adj->values)))
         return static_cast<int>(SpMVError::INVALID_FORMAT);  // host arrays are what gets sharded
     if (adj->num_cols != adj->num_rows) return static_cast<int>(SpMVError::INVALID_DIMENSION);
@@ -73,7 +79,8 @@ int pagerank_multi(const CSRMatrix* adj, const PageRankConfig* config, int n_gpu
         if (everyone) {
             rc = pr_dist_create(comm, &shard, lo, n, exchange, &d);
             if (rc == 0) {
-                rc = pr_dist_run(d, config, fixed_iterations, &results[rank]);
+                if (personalization) rc = pr_dist_set_personalization(d, personalization);
+                if (rc == 0) rc = pr_dist_run(d, config, fixed_iterations, &results[rank]);
                 if (rc == 0 && rank == 0 &&
                     cudaMemcpy(ranks_out, pr_dist_ranks(d), sizeof(float) * static_cast<size_t>(n), cudaMemcpyDeviceToHost) != cudaSuccess) {
                     cudaGetLastError();

@@ -391,9 +391,11 @@ class NativeComm:
 
 
 class NativeShardedPageRank:
-    """spmv_b200_pr_dist_*: this rank's shard (a DeviceCSR with global column ids) of a sharded PageRank."""
+    """spmv_b200_pr_dist_*: this rank's shard (a DeviceCSR with global column ids) of a sharded PageRank.
+    personalization: the FULL personalization vector (n_global non-negative entries, the same on every
+    rank) for personalized PageRank, or None for global PageRank; set_personalization changes it later."""
 
-    def __init__(self, comm, csr, row_offset, n_global, exchange=EXCHANGE_AUTO):
+    def __init__(self, comm, csr, row_offset, n_global, exchange=EXCHANGE_AUTO, personalization=None):
         self.comm, self.csr, self.n = comm, csr, int(n_global)
         self.handle = C.c_void_p()
         rc = sp.lib.spmv_b200_pr_dist_create(comm.handle, csr.ptr, int(row_offset), self.n, int(exchange), C.byref(self.handle))
@@ -401,6 +403,20 @@ class NativeShardedPageRank:
             raise RuntimeError(f"pr_dist_create: {sp.spmv_error_string(rc)}")
         self.exchange = sp.lib.spmv_b200_pr_dist_exchange(self.handle)
         self.hub_columns = sp.lib.spmv_b200_pr_dist_hub_columns(self.handle)
+        if personalization is not None:
+            try:
+                self.set_personalization(personalization)
+            except Exception:
+                self.close()
+                raise
+
+    def set_personalization(self, personalization):
+        """Collective: personalized PageRank from the next run on (None: global PageRank again)."""
+        v = sp._personalization(personalization, self.n)
+        rc = sp.lib.spmv_b200_pr_dist_set_personalization(self.handle, v.ctypes.data_as(sp.capi.c_float_p)
+                                                          if v is not None else None)
+        if rc != 0:
+            raise RuntimeError(f"pr_dist_set_personalization: {sp.spmv_error_string(rc)}")
 
     def run(self, damping=0.85, tolerance=1e-6, max_iterations=100, fixed_iterations=0):
         cfg = sp.make_pagerank_config(damping, tolerance, max_iterations)

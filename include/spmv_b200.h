@@ -544,6 +544,31 @@ SPMV_B200_API int spmv_b200_pagerank_device_history(const spmv_b200_csr* adj,
                                                     float* final_residual, bool* converged,
                                                     float* l2_history, int history_capacity);
 
+/* ---- personalized PageRank ---------------------------------------------------
+ * Teleport, and the redistribution of dangling mass, follow a caller-given non-negative vector
+ * `personalization` (HOST array of num_rows floats) instead of the uniform 1/n: seed-set /
+ * single-source PPR, topic-sensitive or trust-biased ranking.  With v = personalization / sum(v)
+ * (f64 sum in index order, each entry rounded to fp32) one iteration is
+ *     r_new[i] = (d * (A r_old)[i] + (d * D) * v[i]) + (1 - d) * v[i]
+ * D = dangling mass of r_old; every operation rounded separately in fp32.  r_0 = 1/n, the stop
+ * rule, the residuals and the final normalisation are those of the global form.
+ * INVALID_ARGUMENT, before any device work, when an entry is NaN, +-Inf or negative, when the
+ * entries sum to 0, or when adj is NULL.  personalization == NULL: global PageRank (the
+ * uniform vector gives the same ranks to within rounding, not bit for bit). */
+/* as spmv_b200_pagerank: host ranks in out->ranks, release with spmv_b200_pagerank_free */
+SPMV_B200_API int spmv_b200_pagerank_personalized(const spmv_b200_csr* adj,
+                                                  const spmv_b200_pagerank_config* config,
+                                                  const float* personalization,
+                                                  spmv_b200_pagerank_result* out);
+/* as spmv_b200_pagerank_device / _history: ranks stay on the device; l1_residual, l2_history
+ * (history_capacity entries) are optional */
+SPMV_B200_API int spmv_b200_pagerank_device_personalized(const spmv_b200_csr* adj,
+                                                         const spmv_b200_pagerank_config* config,
+                                                         const float* personalization, float* d_ranks,
+                                                         int* iterations, float* final_residual,
+                                                         bool* converged, double* l1_residual,
+                                                         float* l2_history, int history_capacity);
+
 /* ---- multi-GPU PageRank, host side in C++ ---------------------------------
  * The reference has no multi-GPU code.  This is the multi-GPU member of its signature family
  * pagerank(adj, config) -> ranks (reference include/spmv/pagerank.h:29-32, src/pagerank.cu:50-153):
@@ -583,6 +608,14 @@ SPMV_B200_API int spmv_b200_pagerank_multi(const spmv_b200_csr* adj, const spmv_
                                            int n_gpus, const int* devices, int exchange, int row_weight,
                                            int fixed_iterations, float* ranks_out,
                                            spmv_b200_pr_dist_result* out);
+/* spmv_b200_pagerank_multi for personalized PageRank (personalization: host [num_rows], see
+ * spmv_b200_pagerank_personalized; NULL: spmv_b200_pagerank_multi) */
+SPMV_B200_API int spmv_b200_pagerank_multi_personalized(const spmv_b200_csr* adj,
+                                                        const spmv_b200_pagerank_config* config,
+                                                        const float* personalization, int n_gpus,
+                                                        const int* devices, int exchange, int row_weight,
+                                                        int fixed_iterations, float* ranks_out,
+                                                        spmv_b200_pr_dist_result* out);
 
 /* One process PER GPU (torchrun, mpirun, any launcher): a communicator for the set-up traffic
  * (shard bounds, NCCL id, descriptors of the symmetric allocations) over an abstract unix-domain
@@ -604,6 +637,10 @@ SPMV_B200_API int spmv_b200_pr_dist_create(spmv_b200_comm* comm, const spmv_b200
                                            int n_global, int exchange, spmv_b200_pr_dist** out);
 SPMV_B200_API int spmv_b200_pr_dist_run(spmv_b200_pr_dist* d, const spmv_b200_pagerank_config* config,
                                         int fixed_iterations, spmv_b200_pr_dist_result* out);
+/* Personalized PageRank from the next run on (collective): every rank passes the FULL host vector
+ * (n_global floats, the same on every rank; see spmv_b200_pagerank_personalized) and keeps the
+ * normalised entries of its own rows.  NULL returns to global PageRank. */
+SPMV_B200_API int spmv_b200_pr_dist_set_personalization(spmv_b200_pr_dist* d, const float* personalization);
 /* device pointer to the full, normalised rank vector of the last run (identical on every rank) */
 SPMV_B200_API const float* spmv_b200_pr_dist_ranks(const spmv_b200_pr_dist* d);
 SPMV_B200_API int spmv_b200_pr_dist_exchange(const spmv_b200_pr_dist* d);
