@@ -440,6 +440,74 @@ def pagerank_device_personalized(adj_matrix, d_ranks, personalization, config=No
     return rc, it.value, res.value, conv.value, l1.value, hist
 
 
+# ------------------------------------------- batched personalized PageRank (libspmv_b200_ppr.so) ----
+_ppr = None
+
+
+def ppr_lib():
+    """libspmv_b200_ppr.so, loaded on first use: importing the package does not need the companion."""
+    global _ppr
+    if _ppr is None:
+        _ppr = capi.load_ppr()
+    return _ppr
+
+
+def _teleport_columns(V, n):
+    """(k, offsets, nodes, weights) of the sparse column form of V; weights None means all 1."""
+    try:
+        import scipy.sparse as S
+        if S.issparse(V):
+            M = S.csr_matrix(V)
+            if M.ndim != 2 or M.shape[1] != n:
+                raise ValueError(f"a sparse V must be (k, {n}), got {M.shape}")
+            M = M.sorted_indices()
+            return (M.shape[0], np.ascontiguousarray(M.indptr, np.int32), np.ascontiguousarray(M.indices, np.int32),
+                    np.ascontiguousarray(M.data, np.float32))
+    except ImportError:
+        pass
+    V = np.asarray(V)
+    if V.ndim == 1:  # seed node ids: one-hot vectors
+        if V.size and not np.issubdtype(V.dtype, np.integer):
+            raise ValueError("a 1-D V holds seed node ids (integers)")
+        k = V.size
+        return k, np.arange(k + 1, dtype=np.int32), np.ascontiguousarray(V, np.int32), None
+    if V.ndim != 2 or V.shape[1] != n:
+        raise ValueError(f"a dense V must be (k, {n}), got shape {V.shape}")
+    V = np.ascontiguousarray(V, np.float32)
+    rows, cols = np.nonzero(V)  # row-major order: ascending nodes per column; zeros add nothing to the sum
+    offsets = np.zeros(V.shape[0] + 1, np.int32)
+    offsets[1:] = np.cumsum(np.bincount(rows, minlength=V.shape[0]))
+    return V.shape[0], offsets, cols.astype(np.int32), V[rows, cols]
+
+
+def pagerank_personalized_batch(A, V, config=None, capacity=0):
+    """k personalized PageRank vectors of the graph A (device CSR) in one loop.
+
+    V: a 1-D sequence of seed node ids (one-hot teleport vectors), a dense (k, n) array, or a scipy.sparse (k, n)
+    matrix; each row is normalised by the library, as in pagerank_personalized.  Returns (ranks, iterations,
+    residual, converged, history): ranks is an (n, k) float32 torch tensor on the current CUDA device (column c is
+    vector c), the others are per-column numpy arrays; history is (k, capacity), NaN beyond a column's iterations.
+    Raises RuntimeError with the library's status on a rejected input."""
+    import torch
+    lib_p = ppr_lib()
+    n = A.contents.num_rows if A else 0
+    k, offsets, nodes, weights = _teleport_columns(V, n)
+    ranks = torch.empty((n, k), dtype=torch.float32, device=torch.device("cuda", torch.cuda.current_device()))
+    it = np.zeros(k, np.int32)
+    res = np.zeros(k, np.float32)
+    conv = np.zeros(k, np.bool_)
+    hist = np.full((k, capacity), np.nan, dtype=np.float32)
+    cfg = C.byref(config) if config is not None else None
+    rc = lib_p.spmv_b200_pagerank_personalized_batch(
+        A, cfg, k, offsets.ctypes.data_as(capi.c_int_p), nodes.ctypes.data_as(capi.c_int_p),
+        weights.ctypes.data_as(capi.c_float_p) if weights is not None else None, dptr(ranks), it.ctypes.data_as(capi.c_int_p),
+        res.ctypes.data_as(capi.c_float_p), conv.ctypes.data_as(C.POINTER(C.c_bool)),
+        hist.ctypes.data_as(capi.c_float_p) if capacity > 0 else None, capacity)
+    if rc != 0:
+        raise RuntimeError(f"pagerank_personalized_batch: {spmv_error_string(rc)}")
+    return ranks, it, res, conv, hist
+
+
 # --------------------------------------------------------------- benchmark ----
 
 def make_bench_config(num_warmup_runs=5, num_runs=20, compare_cpu=True):

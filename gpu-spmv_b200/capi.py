@@ -209,6 +209,28 @@ PROTOTYPES = {
 }
 
 
+# ---- include/spmv_b200_ppr.h: the companion library libspmv_b200_ppr.so (batched personalized PageRank) ----
+PPR_LIB_PATH = os.path.join(os.path.dirname(LIB_PATH), "libspmv_b200_ppr.so")
+
+PPR_PROTOTYPES = {
+    "spmv_b200_pagerank_personalized_batch": (C.c_int, [CSR_P, PRC_P, C.c_int, c_int_p, c_int_p, c_float_p, C.c_void_p,
+                                                        c_int_p, c_float_p, C.POINTER(C.c_bool), c_float_p, C.c_int]),
+    "spmv_b200_ppr_launch_count": (C.c_ulonglong, []),
+}
+
+
+def load_ppr(path=PPR_LIB_PATH):
+    """dlopen libspmv_b200_ppr.so (it loads libspmv_b200.so from its own directory) and attach prototypes."""
+    if not os.path.exists(path):
+        raise ImportError(f"{path} not found: build it with `make -C gpu-spmv_b200/csrc` (there is no CPU fallback)")
+    lib = C.CDLL(path)
+    for name, (restype, argtypes) in PPR_PROTOTYPES.items():
+        fn = getattr(lib, name)
+        fn.restype = restype
+        fn.argtypes = argtypes
+    return lib
+
+
 def load(path=LIB_PATH):
     """dlopen the library and attach prototypes.  Raises if it is missing:
     there is deliberately no fallback implementation."""
