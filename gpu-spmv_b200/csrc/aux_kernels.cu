@@ -16,6 +16,7 @@ inline unsigned grid_for(long long n, int per_block = kBlock, unsigned cap = 148
     if (b < 1) b = 1;
     return static_cast<unsigned>(b < cap ? b : cap);
 }
+static_assert(kPrScratchDoubles >= 148 * 16, "pr_init and normalize store one double per CTA of grid_for's grid");
 
 // d_colsum[c] += values[j] for every stored entry (find_dangling_nodes, reference
 // src/pagerank.cu:30-40).  The sums are accumulated in f64: an fp32 value enters an f64 sum without
@@ -160,7 +161,7 @@ cudaError_t launch_dangling_bits(const double* d_colsum, int n, int valid_cols, 
     return cudaGetLastError();
 }
 
-// d_tmp: at least 148*16 doubles
+// d_tmp: kPrScratchDoubles doubles
 cudaError_t launch_pr_init(int n, const uint32_t* d_bits, float* d_r, float* d_dsum, double* d_tmp,
                            cudaStream_t stream) {
     if (n <= 0) return cudaSuccess;
@@ -178,7 +179,7 @@ cudaError_t launch_next_dsum(const double* d_partial, float* d_dsum, cudaStream_
     return cudaGetLastError();
 }
 
-// d_tmp: at least 148*16 doubles
+// d_tmp: kPrScratchDoubles doubles
 cudaError_t launch_normalize(const float* d_r, int n, float* d_out, double* d_tmp, cudaStream_t stream) {
     if (n <= 0) return cudaSuccess;
     const unsigned blocks = grid_for(n);

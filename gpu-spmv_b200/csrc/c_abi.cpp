@@ -578,7 +578,7 @@ int spmv_b200_pr_init(int n, const uint32_t* d_bits, float* d_r, float* d_dsum, 
     if (!d_bits || !d_r || !d_dsum || n < 0) return kBadArg;
     return guarded([&] {
         double* tmp = nullptr;
-        CUDA_CHECK(cudaMalloc(&tmp, sizeof(double) * (148 * 16 + 8)));
+        CUDA_CHECK(cudaMalloc(&tmp, sizeof(double) * b200::kPrScratchDoubles));
         const cudaError_t e = b200::launch_pr_init(n, d_bits, d_r, d_dsum, tmp, static_cast<cudaStream_t>(stream));
         cudaStreamSynchronize(static_cast<cudaStream_t>(stream));
         cudaFree(tmp);
@@ -646,7 +646,7 @@ int spmv_b200_pr_normalize(const float* d_r, int n, float* d_out, void* stream) 
     if (!d_r || !d_out || n < 0) return kBadArg;
     return guarded([&] {
         double* tmp = nullptr;
-        CUDA_CHECK(cudaMalloc(&tmp, sizeof(double) * (148 * 16 + 8)));
+        CUDA_CHECK(cudaMalloc(&tmp, sizeof(double) * b200::kPrScratchDoubles));
         const cudaError_t e = b200::launch_normalize(d_r, n, d_out, tmp, static_cast<cudaStream_t>(stream));
         cudaStreamSynchronize(static_cast<cudaStream_t>(stream));
         cudaFree(tmp);

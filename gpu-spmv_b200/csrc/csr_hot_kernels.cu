@@ -443,11 +443,6 @@ __global__ void hot_encode_kernel(int nnz, int cols, const int* __restrict__ col
     }
 }
 
-int hot_env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 int device_sms() {
     int sms = 148, dev_id = 0;
     cudaGetDevice(&dev_id);
@@ -466,7 +461,7 @@ cudaError_t run_hot_variant(const CsrView& A, const HotPlan& hot, const float* x
     if (e != cudaSuccess) return e;
     // L2 priorities (bit 0: stream evict_first, bit 1: x gathers evict_last).  Default: on when x does not
     // fit L2 comfortably (> 64 MB), where the 8 B/nnz stream would otherwise push x out; SPMV_B200_HOT_L2 forces.
-    static const int env_l2 = hot_env_int("SPMV_B200_HOT_L2", -1);
+    static const int env_l2 = env_int("SPMV_B200_HOT_L2", -1);
     const int l2_mode = env_l2 >= 0 ? env_l2 : 0;
     int grid = sms;  // persistent: one CTA per SM
     if (grid > plan.num_tiles / kWorkers) grid = plan.num_tiles / kWorkers;  // per-worker sums fit plan.partials
@@ -515,7 +510,7 @@ int hot_capacity() {
 // misses -- with the 192 KB table ncu shows the data pipe at 48 % and the kernel 50 % slower than
 // with 64-128 KB (profiles/r1_hub_kernel.md).
 int hot_default_capacity() {
-    static const int env_cap = hot_env_int("SPMV_B200_HOT_CAP", 0);
+    static const int env_cap = env_int("SPMV_B200_HOT_CAP", 0);
     const int cap = hot_capacity();
     const int want = env_cap > 0 ? (env_cap & ~3) : 24576;
     return want < cap ? want : cap;

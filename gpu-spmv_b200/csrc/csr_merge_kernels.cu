@@ -331,17 +331,12 @@ reduce_partials_kernel(const double* __restrict__ partials, int count, double* _
     }
 }
 
-int merge_env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 template <class Row>
 cudaError_t run_tiles(const CsrView& A, const float* x, const MergePlan& plan, const Row& row_op,
                       cudaStream_t stream) {
     if (plan.num_tiles <= 0) return cudaSuccess;
-    static const int use_tma = merge_env_int("SPMV_B200_MERGE_TMA", 0);
-    static const int carveout = merge_env_int("SPMV_B200_MERGE_CARVEOUT", -1);
+    static const int use_tma = env_int("SPMV_B200_MERGE_TMA", 0);
+    static const int carveout = env_int("SPMV_B200_MERGE_CARVEOUT", -1);
     auto launch = [&](auto kernel, int ipt) {
         if (carveout >= 0) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
         const size_t dyn_smem = use_tma ? (kT * ipt + 4) * sizeof(int) : 0;
@@ -360,7 +355,7 @@ cudaError_t run_tiles(const CsrView& A, const float* x, const MergePlan& plan, c
 }  // namespace
 
 int merge_items_for(int rows, int nnz) {
-    static const int forced = merge_env_int("SPMV_B200_MERGE_IPT", 0);  // 7 / 8: A/B timing
+    static const int forced = env_int("SPMV_B200_MERGE_IPT", 0);  // 7 / 8: A/B timing
     if (forced == 7 || forced == 8) return forced;
     // measured (scripts/time_mid.py, bench_hot.py; 7 / 8 items): config 2 0.380 / 0.321 ms, 7-point stencil
     // 0.129 / 0.102, 9-point 0.154 / 0.134, random rows avg 5 and 8 equal, avg 12-24 0.271 / 0.273 .. 0.488 / 0.498,

@@ -424,11 +424,6 @@ __global__ void seg_span_heads_kernel(int num_spans, int n_heads, const int* __r
     tile_head_base[t] = lo;
 }
 
-int seg_env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 cudaError_t run_seg(const SegPlan& P, const float* values, const float* x, float* y, cudaStream_t stream) {
     const size_t smem = static_cast<size_t>((P.n_hot + 3) & ~3) * 4 + kSegFixedSmem;
     cudaError_t e = cudaFuncSetAttribute(seg_spmv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
@@ -463,7 +458,7 @@ int seg_table_capacity() {
 // Table size used when the caller does not ask for one.  Not the maximum: shared memory is carved
 // out of the same 256 KB as the L1, whose lines track the outstanding gather misses.
 int seg_default_capacity() {
-    static const int env_cap = seg_env_int("SPMV_B200_HOT_CAP", 0);
+    static const int env_cap = env_int("SPMV_B200_HOT_CAP", 0);
     const int cap = seg_table_capacity();
     const int want = env_cap > 0 ? (env_cap & ~3) : 24576;
     return want < cap ? want : cap;

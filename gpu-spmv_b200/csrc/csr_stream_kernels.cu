@@ -627,11 +627,6 @@ csr_short_kernel(int rows, int nnz, const int* __restrict__ row_ptrs, const int*
     }
 }
 
-int stream_env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 // window = groups * rows_per_group rows holding about 1.5 K non-zeros; cap = stage capacity
 template <int LPR>
 void pipe_geometry(const CsrView& A, int& rpg, int& cap) {
@@ -640,7 +635,7 @@ void pipe_geometry(const CsrView& A, int& rpg, int& cap) {
     // measured on config 2 (profiles/r1_ell_tuning.md): ~1.5 K non-zeros per window for one lane per row,
     // ~2.5 K when lanes share rows (two row slots are walked together there)
     rpg = static_cast<int>((LPR == 1 ? 1536.0 : 2560.0) / (avg * groups) + 0.5);
-    static const int env_rpg = stream_env_int("SPMV_B200_CSR_RPG", 0);
+    static const int env_rpg = env_int("SPMV_B200_CSR_RPG", 0);
     if (env_rpg > 0) rpg = env_rpg;
     rpg = rpg < 1 ? 1 : (rpg > 8 ? 8 : rpg);
     const int window = groups * rpg;
@@ -700,8 +695,8 @@ cudaError_t launch_pipe_lpr_u(const CsrView& A, const float* x, float* y, cudaSt
     int rpg, cap;
     pipe_geometry<LPR>(A, rpg, cap);
     const int window = groups * rpg;
-    static const int env_stages = stream_env_int("SPMV_B200_CSR_STAGES", 0);
-    static const int env_ctas = stream_env_int("SPMV_B200_CSR_CTAS_PER_SM", 0);
+    static const int env_stages = env_int("SPMV_B200_CSR_STAGES", 0);
+    static const int env_ctas = env_int("SPMV_B200_CSR_CTAS_PER_SM", 0);
     const int stages = env_stages > 1 ? (env_stages > 16 ? 16 : env_stages) : 2;
     const size_t stage_bytes = sizeof(PipeStageHeader) + static_cast<size_t>(window + 4) * 4 + static_cast<size_t>(cap) * 8;
     const size_t smem = 128 + stages * stage_bytes;
@@ -731,14 +726,14 @@ cudaError_t launch_pipe_lpr_u(const CsrView& A, const float* x, float* y, cudaSt
 // gathers per batch: enough to cover an average row of the group's lanes in one batch
 template <int LPR>
 cudaError_t launch_pipe_lpr(const CsrView& A, const float* x, float* y, cudaStream_t stream) {
-    static const int env_u = stream_env_int("SPMV_B200_CSR_U", 0);
+    static const int env_u = env_int("SPMV_B200_CSR_U", 0);
     const double per_lane = static_cast<double>(A.nnz) / A.rows / LPR;
     int u = per_lane <= 4.0 ? 4 : (per_lane <= 6.0 ? 6 : 8);
     if (env_u > 0) u = env_u;
     // a row that takes more than half a stage means windows that do not fit: robust variant
     int rpg, cap;
     pipe_geometry<LPR>(A, rpg, cap);
-    static const int env_robust = stream_env_int("SPMV_B200_CSR_ROBUST", -1);
+    static const int env_robust = env_int("SPMV_B200_CSR_ROBUST", -1);
     const bool robust = env_robust >= 0 ? env_robust != 0 : longest_row_cached(A, stream) > cap / 2;
     if (robust) {
         if (u <= 4) return launch_pipe_lpr_u<LPR, 4, true>(A, x, y, stream);
@@ -755,7 +750,7 @@ cudaError_t launch_short_as(const CsrView& A, const float* x, float* y, cudaStre
     constexpr int S = 2;  // ring depth: deeper rings leave fewer CTAs per SM (measured: 3 stages 0.166 ms against 0.144 ms)
     auto kernel = csr_short_kernel<U, RPT, CAP, S>;
     const size_t smem = 128 + S * sizeof(ShortStage<RPT, CAP>);
-    static const int env_ctas = stream_env_int("SPMV_B200_CSR_CTAS_PER_SM", 0);
+    static const int env_ctas = env_int("SPMV_B200_CSR_CTAS_PER_SM", 0);
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     int fit = 1;
@@ -789,7 +784,7 @@ cudaError_t launch_short(const CsrView& A, const float* x, float* y, cudaStream_
 // Short rows only: a row is walked by one thread, and a window that does not fit a stage is walked
 // from global memory by 256 threads -- both fine while no row is long.
 bool short_eligible(const CsrView& A, cudaStream_t stream) {
-    static const int mode = stream_env_int("SPMV_B200_CSR_SHORT", -1);  // 0 off, 1 forced, -1 by structure
+    static const int mode = env_int("SPMV_B200_CSR_SHORT", -1);  // 0 off, 1 forced, -1 by structure
     if (mode == 0) return false;
     if (mode == 1) return true;
     const double avg = static_cast<double>(A.nnz) / A.rows;
@@ -803,7 +798,7 @@ bool short_eligible(const CsrView& A, cudaStream_t stream) {
 }
 
 bool pipe_eligible(const CsrView& A) {
-    static const int disable = stream_env_int("SPMV_B200_CSR_NO_PIPE", 0);
+    static const int disable = env_int("SPMV_B200_CSR_NO_PIPE", 0);
     const uintptr_t bits = reinterpret_cast<uintptr_t>(A.values) | reinterpret_cast<uintptr_t>(A.col_indices) |
                            reinterpret_cast<uintptr_t>(A.row_ptrs);
     return !disable && (bits & 15u) == 0;
@@ -880,7 +875,7 @@ cudaError_t launch_csr_warp_per_row(const CsrView& A, const float* x, float* y, 
 // with two lanes.  The selector only sends matrices with max <= 10 * (min + 1) here, so no lane is
 // left alone with a long row.  SPMV_B200_VECTOR_LANES forces a width (A/B timing).
 int vector_lanes_for(int rows, int nnz) {
-    static const int forced = stream_env_int("SPMV_B200_VECTOR_LANES", 0);
+    static const int forced = env_int("SPMV_B200_VECTOR_LANES", 0);
     if (forced == 1 || forced == 2 || forced == 4 || forced == 8 || forced == 16 || forced == 32) return forced;
     const double avg = rows > 0 ? static_cast<double>(nnz) / rows : 0.0;
     // measured on 4 M-row matrices (scripts/time_mid.py), one lane against the old choice of 2 / 4 / 8 lanes:

@@ -271,21 +271,17 @@ struct AutoEntry {
 };
 std::mutex g_auto_mu;
 std::unordered_map<const void*, AutoEntry*> g_auto;
+}  // namespace
 
 int hot_env_mode() {
-    static const int mode = [] {
-        const char* v = getenv("SPMV_B200_HOT");
-        return v ? atoi(v) : -1;
-    }();
+    static const int mode = env_int("SPMV_B200_HOT", -1);
     return mode;
 }
-}  // namespace
 
 bool auto_plan_enabled() {
     int v = g_auto_plan_enabled.load(std::memory_order_relaxed);
     if (v < 0) {
-        const char* e = getenv("SPMV_B200_AUTO_PLAN");
-        v = (e && atoi(e) > 0) ? 1 : 0;
+        v = env_int("SPMV_B200_AUTO_PLAN", 0) > 0 ? 1 : 0;
         g_auto_plan_enabled.store(v, std::memory_order_relaxed);
     }
     return v > 0;

@@ -327,11 +327,6 @@ ell_tma_pipe_kernel(int rows, int width, int stages, const int* __restrict__ col
     }
 }
 
-int env_int(const char* name, int fallback) {
-    const char* s = getenv(name);
-    return s ? atoi(s) : fallback;
-}
-
 template <int RPT>
 cudaError_t launch_tma_pipe(int rows, int width, const int* ci, const float* va, const float* x, float* y,
                             unsigned long long* counter, cudaStream_t stream, int row_lo = 0, int row_hi = -1) {
@@ -379,10 +374,7 @@ cudaError_t launch_tma_pipe(int rows, int width, const int* ci, const float* va,
 // 4 / 5 / 6 = persistent TMA pipeline with 4 / 2 / 1 rows per thread.
 // (SPMV_B200_ELL_VARIANT exists for A/B timing on the device; see profiles/.)
 int ell_variant_override() {
-    static const int v = [] {
-        const char* s = getenv("SPMV_B200_ELL_VARIANT");
-        return s ? atoi(s) : 0;
-    }();
+    static const int v = env_int("SPMV_B200_ELL_VARIANT", 0);
     return v;
 }
 

@@ -79,15 +79,10 @@ __global__ void ell_chunk_col_range_kernel(int rows, int width, const int* __res
     }
 }
 
-int env_or(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 // the device address of a page-locked, device-mapped host buffer (nullptr: y_host is something else, or
 // SPMV_B200_HOST_ZERO_COPY_Y=0)
 float* mapped_device_pointer(float* y_host) {
-    static const int zero_copy = env_or("SPMV_B200_HOST_ZERO_COPY_Y", 1);
+    static const int zero_copy = env_int("SPMV_B200_HOST_ZERO_COPY_Y", 1);
     if (!zero_copy) return nullptr;
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, y_host) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
@@ -182,7 +177,7 @@ int ell_host_plan_create(const ELLMatrix* A, int chunks, EllHostPlan** out) {
     // x travels in chunks of the same size as the rows.  (Measured: finer x chunks -- 4 or 8 per row chunk, so that
     // a banded row chunk waits for less beyond its own rows -- cost more in per-copy overhead than they gain:
     // 2.09 / 2.31 ms against 1.83 ms; SPMV_B200_HOST_X_SPLIT keeps the experiment reproducible.)
-    static const int x_per_row_chunk = [] { const char* v = getenv("SPMV_B200_HOST_X_SPLIT"); const int k = v ? atoi(v) : 1; return k < 1 ? 1 : (k > 16 ? 16 : k); }();
+    static const int x_per_row_chunk = std::min(16, std::max(1, env_int("SPMV_B200_HOST_X_SPLIT", 1)));
     const long long xc = static_cast<long long>(chunks) * x_per_row_chunk;
     p->x_chunk = static_cast<int>(std::max<long long>(1024, round_up((static_cast<long long>(p->cols) + xc - 1) / xc, 1024)));
     p->x_chunks = p->cols > 0 ? (p->cols + p->x_chunk - 1) / p->x_chunk : 0;
@@ -227,7 +222,7 @@ int ell_host_plan_create(const ELLMatrix* A, int chunks, EllHostPlan** out) {
         cudaFree(d_max);
     }
     // gated form: per-window poll table, completion flag, progress counters, abort words, second download stream
-    if (ok && p->ranged && env_or("SPMV_B200_HOST_GATED", 1) && write_value32() &&
+    if (ok && p->ranged && env_int("SPMV_B200_HOST_GATED", 1) && write_value32() &&
         ell_gated_applies(p->rows, p->width, p->d_cols, p->d_vals)) {
         const int windows = ell_gated_windows(p->rows);
         // Download chunks: equal ones.  Every D2H copy costs ~19 us of idle down-link on B200 (its completion is a PCIe
@@ -235,7 +230,7 @@ int ell_host_plan_create(const ELLMatrix* A, int chunks, EllHostPlan** out) {
         // 1.640 / 1.669 / 1.683 ms on config 2; a small first chunk followed by growing ones (the download is the
         // slower direction) was measured too and loses to 8 equal chunks (1.71-1.96 ms) -- profiles/r2_host_gated.txt
         {
-            const int want = std::min(255, std::max(1, env_or("SPMV_B200_HOST_GATED_CHUNKS", 8)));
+            const int want = std::min(255, std::max(1, env_int("SPMV_B200_HOST_GATED_CHUNKS", 8)));
             const int size = (windows + want - 1) / want;
             p->g_first.assign(1, 0);
             while (p->g_first.back() < windows) p->g_first.push_back(std::min(windows, p->g_first.back() + size));
@@ -301,9 +296,9 @@ namespace {
 // The gated form.  0: y is complete; 1: the kernel gave up waiting (nothing usable in y: the caller runs the
 // chunked form and stops using this one); < 0: CUDA error.
 int run_gated(EllHostPlan* p, const float* x_host, float* y_host) {
-    static const int down_streams = std::min(2, std::max(1, env_or("SPMV_B200_HOST_DOWN_STREAMS", 1)));
-    static const unsigned long long timeout_ns = 1000000ull * static_cast<unsigned long long>(std::max(1, env_or("SPMV_B200_HOST_GATED_TIMEOUT_MS", 2000)));
-    static const unsigned poll_sleep_ns = static_cast<unsigned>(std::max(0, env_or("SPMV_B200_HOST_GATED_POLL_NS", 200)));
+    static const int down_streams = std::min(2, std::max(1, env_int("SPMV_B200_HOST_DOWN_STREAMS", 1)));
+    static const unsigned long long timeout_ns = 1000000ull * static_cast<unsigned long long>(std::max(1, env_int("SPMV_B200_HOST_GATED_TIMEOUT_MS", 2000)));
+    static const unsigned poll_sleep_ns = static_cast<unsigned>(std::max(0, env_int("SPMV_B200_HOST_GATED_POLL_NS", 200)));
     static const bool trace = getenv("SPMV_B200_TRACE") != nullptr;
     const StreamValue32Fn write32 = write_value32();
     const unsigned epoch = ++p->epoch == 0 ? ++p->epoch : p->epoch;  // flags start at 0: never a valid epoch
@@ -320,7 +315,7 @@ int run_gated(EllHostPlan* p, const float* x_host, float* y_host) {
     ok = ok && cudaStreamWaitEvent(p->s_up, p->ev_fill, 0) == cudaSuccess;
     // SPMV_B200_HOST_GATED_TEST_STALL=1 (tests only): the upload never happens, so the kernel must time out, drain and hand the
     // call to the chunked form -- the path that guarantees the call cannot hang
-    static const int test_stall = env_or("SPMV_B200_HOST_GATED_TEST_STALL", 0);
+    static const int test_stall = env_int("SPMV_B200_HOST_GATED_TEST_STALL", 0);
     if (ok && p->up_hi > p->up_lo && !test_stall)
         ok = cudaMemcpyAsync(p->d_x + p->up_lo, x_host + p->up_lo, (p->up_hi - p->up_lo) * sizeof(float), cudaMemcpyHostToDevice, p->s_up) == cudaSuccess;
     if (!test_stall) ok = ok && write32(reinterpret_cast<CUstream>(p->s_up), reinterpret_cast<CUdeviceptr>(p->d_done), epoch, 0) == CUDA_SUCCESS;

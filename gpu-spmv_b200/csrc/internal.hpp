@@ -7,10 +7,20 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <cstdlib>
+#include <functional>
 #include <vector>
 
 namespace spmv {
 namespace b200 {
+
+// ---- environment ------------------------------------------------------------------
+// atoi of environment variable `name`, or `fallback` when it is unset.  Callers keep the result in a
+// function-local static where a variable is read once per process.
+inline int env_int(const char* name, int fallback) {
+    const char* v = std::getenv(name);
+    return v ? std::atoi(v) : fallback;
+}
 
 // ---- selector -----------------------------------------------------------------
 // A SCALAR_CSR decision is overridden to MERGE_PATH when a row is longer than
@@ -233,6 +243,8 @@ struct PlannedCsr {
 // prefer_seg: take the segmented stream first when rows average >= 4 non-zeros (single-shard PageRank).
 cudaError_t planned_build(const CsrView& A, PlannedCsr* out, int capacity, bool force, bool allow_seg,
                           cudaStream_t stream, bool prefer_seg = false);
+// SPMV_B200_HOT: 0 no hub-column / segmented plans, > 0 plans without the size / benefit thresholds, -1 (unset) by structure
+int hot_env_mode();
 // out[3] = ordered sum of `count` triples of per-CTA partial sums
 cudaError_t launch_reduce_partials(const double* partials, int count, double* out, cudaStream_t stream);
 
@@ -240,6 +252,8 @@ cudaError_t launch_reduce_partials(const double* partials, int count, double* ou
 cudaError_t launch_colsum(const CsrView& A, double* d_colsum, cudaStream_t stream);  // f64 sums: see aux_kernels.cu
 cudaError_t launch_dangling_bits(const double* d_colsum, int n, int valid_cols, uint32_t* d_bits,
                                  cudaStream_t stream);
+// d_tmp of launch_pr_init and launch_normalize: one double per CTA of their grids (at most 148 * 16)
+constexpr int kPrScratchDoubles = 148 * 16 + 8;
 cudaError_t launch_pr_init(int n, const uint32_t* d_bits, float* d_r, float* d_dsum,
                            double* d_tmp, cudaStream_t stream);
 cudaError_t launch_next_dsum(const double* d_partial, float* d_dsum, cudaStream_t stream);
@@ -317,6 +331,30 @@ int pr_step(PrPlan* plan, const float* d_r_old, float* d_r_new, float damping, c
 const CsrView& pr_plan_view(const PrPlan* plan);
 int pr_plan_hub_columns(const PrPlan* plan);  // entries of the shared-memory x table in use (0: none)
 double* pr_plan_tmp(PrPlan* plan);
+// Dangling bitmask of a whole graph (A.rows == A.cols): zeroes d_colsum [A.cols], sums the columns into it in f64 and
+// sets bit c where column c sums to 0 (reference src/pagerank.cu:20-48).
+cudaError_t pr_dangling_bits(const CsrView& A, double* d_colsum, uint32_t* d_bits, cudaStream_t stream);
+
+// CUDA graphs of the two ping-pong iterations of a PageRank loop (p = 0: vector a -> b, p = 1: b -> a), captured
+// once and replayed: one graph launch per iteration instead of one API call per kernel and copy, where small graphs
+// are launch-bound.  SPMV_B200_PR_GRAPH=0 disables them.
+struct PrIterationGraphs {
+    cudaGraphExec_t exec[2] = {nullptr, nullptr};
+    unsigned long long launches_per_iteration = 0;  // launches one replay stands for (set by capture)
+    PrIterationGraphs() = default;
+    PrIterationGraphs(const PrIterationGraphs&) = delete;
+    PrIterationGraphs& operator=(const PrIterationGraphs&) = delete;
+    ~PrIterationGraphs() { reset(); }
+    // capturing pays off for a loop of this many iterations (and SPMV_B200_PR_GRAPH allows it)
+    static bool wanted(int iterations);
+    bool ready() const { return exec[0] && exec[1]; }
+    // enqueue(p) enqueues iteration p on `stream` and returns 0.  On any failure no graph is kept, false is
+    // returned, and launch_count() is what it was before the call.
+    bool capture(cudaStream_t stream, const std::function<int(int)>& enqueue);
+    // replays iteration p and counts its launches
+    bool launch(int p, cudaStream_t stream);
+    void reset();
+};
 // d_pvec: the normalised personalization vector [n] on the device (pr_personalization_upload), or nullptr
 int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d_ranks, int* iterations,
                     float* final_residual, bool* converged, double* l1_residual, bool normalize = true, float* l2_history = nullptr, int history_capacity = 0,

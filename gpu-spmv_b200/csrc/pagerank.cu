@@ -21,13 +21,10 @@
 #include "internal.hpp"
 
 #include <cmath>
-#include <cstdlib>
 #include <new>
 
 namespace spmv {
 namespace b200 {
-
-constexpr int kTmpDoubles = 148 * 16 + 8;
 
 // A plan over one row shard: merge-path coordinates are computed once (the
 // matrix is constant across iterations) and the work arrays are owned here.
@@ -37,7 +34,7 @@ struct PrPlan {
     int n_global = 0;
     Scratch merge_block;
     MergePlan merge;
-    Scratch tmp_block;   // kTmpDoubles doubles
+    Scratch tmp_block;   // kPrScratchDoubles doubles
     double* tmp = nullptr;
     // A ROW SHARD of a scale-free graph takes the hub-column plan: the tile epilogue of that kernel
     // overlaps the slice exchange with the product (8 GPUs, R-MAT 26: 1.17 vs 1.46 ms per iteration
@@ -48,14 +45,6 @@ struct PrPlan {
     bool whole_graph = false;
     ~PrPlan() { planned.release(); }
 };
-
-static int pr_hot_env() {
-    static const int mode = [] {
-        const char* v = getenv("SPMV_B200_HOT");
-        return v ? atoi(v) : -1;
-    }();
-    return mode;
-}
 
 int pr_plan_create(const CSRMatrix* shard, int row_offset, int n_global, cudaStream_t stream, PrPlan** out) {
     if (!shard || !out || row_offset < 0 || n_global < 0) return static_cast<int>(SpMVError::INVALID_ARGUMENT);
@@ -73,7 +62,7 @@ int pr_plan_create(const CSRMatrix* shard, int row_offset, int n_global, cudaStr
     p->row_offset = row_offset;
     p->n_global = n_global;
     void* block = p->merge_block.reserve(merge_plan_bytes(p->A.rows, p->A.nnz, true));
-    p->tmp = static_cast<double*>(p->tmp_block.reserve(kTmpDoubles * sizeof(double)));
+    p->tmp = static_cast<double*>(p->tmp_block.reserve(kPrScratchDoubles * sizeof(double)));
     if (!block || !p->tmp) {
         delete p;
         return static_cast<int>(SpMVError::CUDA_MALLOC);
@@ -86,8 +75,8 @@ int pr_plan_create(const CSRMatrix* shard, int row_offset, int n_global, cudaStr
     }
     // the matrix is constant over the iterations: the hub-column plan pays for itself after a few
     p->whole_graph = row_offset == 0 && shard->num_rows == n_global;
-    if (pr_hot_env() != 0 &&
-        planned_build(p->A, &p->planned, 0, pr_hot_env() > 0, p->whole_graph, stream, p->whole_graph) != cudaSuccess) {
+    if (hot_env_mode() != 0 &&
+        planned_build(p->A, &p->planned, 0, hot_env_mode() > 0, p->whole_graph, stream, p->whole_graph) != cudaSuccess) {
         cudaGetLastError();
         p->planned.release();  // not fatal: the plain tile kernel is used
     }
@@ -152,6 +141,56 @@ int pr_plan_hub_columns(const PrPlan* p) {
 }
 double* pr_plan_tmp(PrPlan* p) { return p->tmp; }
 
+cudaError_t pr_dangling_bits(const CsrView& A, double* d_colsum, uint32_t* d_bits, cudaStream_t stream) {
+    cudaError_t e = cudaMemsetAsync(d_colsum, 0, sizeof(double) * A.cols, stream);
+    if (e == cudaSuccess) e = launch_colsum(A, d_colsum, stream);
+    if (e == cudaSuccess) e = launch_dangling_bits(d_colsum, A.cols, A.cols, d_bits, stream);
+    return e;
+}
+
+bool PrIterationGraphs::wanted(int iterations) {
+    static const int enabled = env_int("SPMV_B200_PR_GRAPH", 1);
+    return enabled && iterations >= 4;
+}
+
+bool PrIterationGraphs::capture(cudaStream_t stream, const std::function<int(int)>& enqueue) {
+    for (int p = 0; p < 2; ++p) {
+        cudaGraph_t g = nullptr;
+        const unsigned long long before = launch_count();
+        bool good = cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
+        if (good) {
+            const int r = enqueue(p);
+            good = cudaStreamEndCapture(stream, &g) == cudaSuccess && r == 0 && g != nullptr;
+        }
+        launches_per_iteration = launch_count() - before;
+        count_launches(-static_cast<int>(launches_per_iteration));  // captured, not launched
+        if (good) good = cudaGraphInstantiate(&exec[p], g, 0) == cudaSuccess;
+        if (g) cudaGraphDestroy(g);
+        if (!good) {
+            cudaGetLastError();
+            reset();
+            return false;
+        }
+    }
+    return true;
+}
+
+bool PrIterationGraphs::launch(int p, cudaStream_t stream) {
+    if (cudaGraphLaunch(exec[p], stream) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    count_launches(static_cast<int>(launches_per_iteration));
+    return true;
+}
+
+void PrIterationGraphs::reset() {
+    for (int p = 0; p < 2; ++p) {
+        if (exec[p]) cudaGraphExecDestroy(exec[p]);
+        exec[p] = nullptr;
+    }
+}
+
 // pagerank_small.cu
 bool pagerank_small_applies(int n, int nnz);
 cudaError_t pagerank_small_run(const CsrView& A, float damping, float tolerance, int max_iterations, const uint32_t* d_bits,
@@ -159,55 +198,50 @@ cudaError_t pagerank_small_run(const CsrView& A, float damping, float tolerance,
                                int* iterations, float* residual, double* l1, bool* converged, int* final_buffer,
                                cudaStream_t stream, const float* d_pvec);
 
-// The loop of a small graph in one persistent kernel (pagerank_small.cu); same set-up, same outputs as the
-// multi-kernel loop below.  kNotHandled: take that loop instead.
-constexpr int kNotHandled = 1 << 20;
-static int pagerank_device_small(const CSRMatrix* adj, const PageRankConfig* config, float* d_ranks, int* iterations,
-                                 float* final_residual, bool* converged, double* l1_residual, bool normalize, float* l2_history,
-                                 int history_capacity, const float* d_pvec) {
-    const int n = adj->num_rows;
-    if (!adj->d_row_ptrs || (adj->nnz > 0 && (!adj->d_col_indices || !adj->d_values))) return kNotHandled;  // the loop below reports it
-    const CsrView A = view_of(adj);
-    cudaStream_t stream = nullptr;
-    const size_t words = (static_cast<size_t>(n) + 31) / 32;
-    float *d_a = nullptr, *d_b = nullptr, *d_dsum = nullptr;
-    double *d_colsum = nullptr, *d_tmp = nullptr;
-    uint32_t* d_bits = nullptr;
-    const bool ok = cudaMalloc(&d_a, sizeof(float) * n) == cudaSuccess && cudaMalloc(&d_b, sizeof(float) * n) == cudaSuccess &&
-                    cudaMalloc(&d_colsum, sizeof(double) * n) == cudaSuccess && cudaMalloc(&d_bits, sizeof(uint32_t) * words) == cudaSuccess &&
-                    cudaMalloc(&d_dsum, sizeof(float)) == cudaSuccess && cudaMalloc(&d_tmp, sizeof(double) * kTmpDoubles) == cudaSuccess;
-    int rc = 0;
-    if (!ok) {
-        cudaGetLastError();
-        rc = static_cast<int>(SpMVError::CUDA_MALLOC);
-    } else {
-        // dangling nodes, r = 1/n and its dangling mass: exactly as below
-        cudaMemsetAsync(d_colsum, 0, sizeof(double) * n, stream);
-        launch_colsum(A, d_colsum, stream);
-        launch_dangling_bits(d_colsum, n, n, d_bits, stream);
-        launch_pr_init(n, d_bits, d_a, d_dsum, d_tmp, stream);
-        int fin = 0;
-        const cudaError_t e = pagerank_small_run(A, config->damping_factor, config->tolerance, config->max_iterations, d_bits, d_a, d_b,
-                                                 d_dsum, l2_history, history_capacity, iterations, final_residual, l1_residual,
-                                                 converged, &fin, stream, d_pvec);
-        if (e == cudaErrorNotSupported) {
-            rc = kNotHandled;
-        } else if (e != cudaSuccess) {
-            cudaGetLastError();
-            rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
-        } else {
-            const float* vec = fin ? d_b : d_a;
-            if (normalize) launch_normalize(vec, n, d_ranks, d_tmp, stream);
-            else cudaMemcpyAsync(d_ranks, vec, sizeof(float) * n, cudaMemcpyDeviceToDevice, stream);
-            if (cudaStreamSynchronize(stream) != cudaSuccess) {
-                cudaGetLastError();
-                rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
-            }
-        }
+// What one single-GPU run allocates, freed on every return.  init() sets up what both loops start from; the
+// multi-kernel loop adds its plan and the two copies of the per-iteration sums.
+struct PrRun {
+    float *a = nullptr, *b = nullptr;  // the rank vectors; a holds r_0
+    double* colsum = nullptr;
+    uint32_t* bits = nullptr;          // dangling bitmask
+    float* dsum = nullptr;             // dangling mass of r_0
+    double* tmp = nullptr;             // kPrScratchDoubles, for pr_init and normalize
+    PrPlan* plan = nullptr;
+    double* partial = nullptr;         // device {sum d^2, sum |d|, dangling mass} of one iteration
+    double* h_partial = nullptr;       // pinned, one triple per ping-pong slot
+    PrRun() = default;
+    PrRun(const PrRun&) = delete;
+    PrRun& operator=(const PrRun&) = delete;
+    ~PrRun() {
+        cudaFree(a); cudaFree(b); cudaFree(colsum); cudaFree(bits); cudaFree(dsum); cudaFree(tmp); cudaFree(partial);
+        if (h_partial) cudaFreeHost(h_partial);
+        pr_plan_destroy(plan);
     }
-    cudaFree(d_a); cudaFree(d_b); cudaFree(d_colsum); cudaFree(d_bits); cudaFree(d_dsum); cudaFree(d_tmp);
-    return rc;
-}
+    // dangling nodes, r_0 = 1/n and its dangling mass (reference :20-48, :69-72, :87, :94-99 for iteration 0)
+    int init(const CsrView& A, cudaStream_t stream) {
+        const int n = A.rows;
+        const size_t words = (static_cast<size_t>(n) + 31) / 32;
+        if (cudaMalloc(&a, sizeof(float) * n) != cudaSuccess || cudaMalloc(&b, sizeof(float) * n) != cudaSuccess ||
+            cudaMalloc(&colsum, sizeof(double) * n) != cudaSuccess || cudaMalloc(&bits, sizeof(uint32_t) * words) != cudaSuccess ||
+            cudaMalloc(&dsum, sizeof(float)) != cudaSuccess || cudaMalloc(&tmp, sizeof(double) * kPrScratchDoubles) != cudaSuccess) {
+            cudaGetLastError();
+            return static_cast<int>(SpMVError::CUDA_MALLOC);
+        }
+        if (pr_dangling_bits(A, colsum, bits, stream) != cudaSuccess || launch_pr_init(n, bits, a, dsum, tmp, stream) != cudaSuccess) {
+            cudaGetLastError();
+            return static_cast<int>(SpMVError::KERNEL_LAUNCH);
+        }
+        return 0;
+    }
+    // final vector (:135-139) into d_ranks, normalised (:142-150) or raw; the stream is synchronised
+    int write_ranks(const float* fin, int n, bool normalize, float* d_ranks, cudaStream_t stream) {
+        if (normalize) launch_normalize(fin, n, d_ranks, tmp, stream);
+        else cudaMemcpyAsync(d_ranks, fin, sizeof(float) * n, cudaMemcpyDeviceToDevice, stream);
+        if (cudaStreamSynchronize(stream) == cudaSuccess) return 0;
+        cudaGetLastError();
+        return static_cast<int>(SpMVError::KERNEL_LAUNCH);
+    }
+};
 
 // The whole loop on one device; d_ranks receives the ranks, normalised on the device with an
 // f64 sum when `normalize` is set, else the raw final iterate.
@@ -227,50 +261,34 @@ int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d
     // non-square adjacency: the reference's first spmv_csr(adj, ..., vec_size = n) fails with INVALID_DIMENSION and
     // pagerank() returns the uniform vector with iterations = 0 (src/pagerank.cu:102-107); pagerank() below does the same
     if (adj->num_cols != n) return static_cast<int>(SpMVError::INVALID_DIMENSION);
-
-    if (pagerank_small_applies(n, adj->nnz)) {  // launch-bound sizes: the whole loop in one persistent kernel
-        const int r = pagerank_device_small(adj, config, d_ranks, iterations, final_residual, converged, l1_residual, normalize,
-                                            l2_history, history_capacity, d_pvec);
-        if (r != kNotHandled) return r;
-    }
+    if (!adj->d_row_ptrs || (adj->nnz > 0 && (!adj->d_col_indices || !adj->d_values)))
+        return static_cast<int>(SpMVError::INVALID_FORMAT);
 
     cudaStream_t stream = nullptr;
-    PrPlan* plan = nullptr;
-    int rc = pr_plan_create(adj, 0, n, stream, &plan);
+    PrRun run;
+    int rc = run.init(view_of(adj), stream);
     if (rc != 0) return rc;
 
-    const int cols = adj->num_cols;
-    const size_t colsum_n = static_cast<size_t>(cols > n ? cols : n);
-    const size_t words = (static_cast<size_t>(n) + 31) / 32;
-    float *d_a = nullptr, *d_b = nullptr, *d_dsum = nullptr;
-    double* d_colsum = nullptr;
-    uint32_t* d_bits = nullptr;
-    double* d_partial = nullptr;
-    double* h_partial = nullptr;
-    bool ok = cudaMalloc(&d_a, sizeof(float) * n) == cudaSuccess &&
-              cudaMalloc(&d_b, sizeof(float) * n) == cudaSuccess &&
-              cudaMalloc(&d_colsum, sizeof(double) * colsum_n) == cudaSuccess &&
-              cudaMalloc(&d_bits, sizeof(uint32_t) * words) == cudaSuccess &&
-              cudaMalloc(&d_dsum, sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&d_partial, 3 * sizeof(double)) == cudaSuccess &&
-              cudaMallocHost(&h_partial, 6 * sizeof(double)) == cudaSuccess;
-    auto cleanup = [&]() {
-        cudaFree(d_a); cudaFree(d_b); cudaFree(d_colsum); cudaFree(d_bits); cudaFree(d_dsum); cudaFree(d_partial);
-        if (h_partial) cudaFreeHost(h_partial);
-        pr_plan_destroy(plan);
-    };
-    if (!ok) {
-        cudaGetLastError();
-        cleanup();
-        return static_cast<int>(SpMVError::CUDA_MALLOC);
+    if (pagerank_small_applies(n, adj->nnz)) {  // launch-bound sizes: the whole loop in one persistent kernel
+        int fin = 0;
+        const cudaError_t e = pagerank_small_run(view_of(adj), config->damping_factor, config->tolerance, config->max_iterations,
+                                                 run.bits, run.a, run.b, run.dsum, l2_history, history_capacity, iterations,
+                                                 final_residual, l1_residual, converged, &fin, stream, d_pvec);
+        if (e == cudaSuccess) return run.write_ranks(fin ? run.b : run.a, n, normalize, d_ranks, stream);
+        if (e != cudaErrorNotSupported) {
+            cudaGetLastError();
+            return static_cast<int>(SpMVError::KERNEL_LAUNCH);
+        }
+        // no cooperative launch on this device: the multi-kernel loop below, on the same (untouched) buffers
     }
 
-    // dangling nodes: columns whose stored values sum to 0 (reference :20-48, :87)
-    cudaMemsetAsync(d_colsum, 0, sizeof(double) * colsum_n, stream);
-    launch_colsum(plan->A, d_colsum, stream);
-    launch_dangling_bits(d_colsum, n, cols, d_bits, stream);
-    // r = 1/n and its dangling mass (reference :69-72, :94-99 for iteration 0)
-    launch_pr_init(n, d_bits, d_a, d_dsum, plan->tmp, stream);
+    rc = pr_plan_create(adj, 0, n, stream, &run.plan);
+    if (rc != 0) return rc;
+    if (cudaMalloc(&run.partial, 3 * sizeof(double)) != cudaSuccess ||
+        cudaMallocHost(&run.h_partial, 6 * sizeof(double)) != cudaSuccess) {
+        cudaGetLastError();
+        return static_cast<int>(SpMVError::CUDA_MALLOC);
+    }
 
     // The stop rule is the reference's (L2 norm of the delta < tolerance, every iteration,
     // :118-127) but it is read one iteration late: the 24-byte sums of iteration i go to pinned
@@ -278,8 +296,8 @@ int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d
     // device never idles on the host.  If iteration i had converged, its output is the INPUT of
     // the speculative iteration i+1 (which writes the other buffer), so vector, iteration count
     // and residual are exactly those of the eager rule.
-    float* r_old = d_a;
-    float* r_new = d_b;
+    float* r_old = run.a;
+    float* r_new = run.b;
     const float* fin = r_old;  // what the reference returns when the loop never runs (:135-139)
     int iters = 0;
     float residual = 0.0f;
@@ -295,8 +313,8 @@ int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d
             rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
             return true;
         }
-        residual = std::sqrt(static_cast<float>(h_partial[3 * p.slot + 0]));  // L2 norm of the delta (:118)
-        l1 = h_partial[3 * p.slot + 1];
+        residual = std::sqrt(static_cast<float>(run.h_partial[3 * p.slot + 0]));  // L2 norm of the delta (:118)
+        l1 = run.h_partial[3 * p.slot + 1];
         iters = p.iter;
         if (l2_history && p.iter >= 1 && p.iter <= history_capacity) l2_history[p.iter - 1] = residual;
         fin = p.vec;
@@ -304,59 +322,29 @@ int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d
     };
     // One iteration = the fused step (3-4 kernels), the dangling-mass hand-over and the 24-byte download.
     auto enqueue_iteration = [&](float* from, float* to, int slot, cudaStream_t s) -> int {
-        const int r = pr_step(plan, from, to, config->damping_factor, d_dsum, d_bits, d_partial, s, nullptr, 0, 0, nullptr,
-                              d_pvec);
+        const int r = pr_step(run.plan, from, to, config->damping_factor, run.dsum, run.bits, run.partial, s, nullptr, 0, 0,
+                              nullptr, d_pvec);
         if (r != 0) return r;
-        launch_next_dsum(d_partial, d_dsum, s);
-        cudaMemcpyAsync(h_partial + 3 * slot, d_partial, 3 * sizeof(double), cudaMemcpyDeviceToHost, s);
+        launch_next_dsum(run.partial, run.dsum, s);
+        cudaMemcpyAsync(run.h_partial + 3 * slot, run.partial, 3 * sizeof(double), cudaMemcpyDeviceToHost, s);
         return 0;
     };
-    // CUDA-graph replay (SURVEY 8f rank 3): the two ping-pong iterations (a -> b with host slot 0,
-    // b -> a with slot 1) are captured once and replayed, one graph launch per iteration instead of
-    // 5-6 API calls -- small graphs are launch-bound.  The stop rule stays per iteration (above).
-    // Capture needs a real stream; a blocking one keeps the legacy default stream's ordering.  Any
-    // failure falls back to the eager loop.  SPMV_B200_PR_GRAPH=0 disables it.
+    // Graph replay (SURVEY 8f rank 3); the stop rule stays per iteration (above).  Capture needs a real
+    // stream; a blocking one keeps the legacy default stream's ordering.  Any failure falls back to the
+    // eager loop.
     cudaStream_t gs = nullptr;
-    cudaGraphExec_t exec[2] = {nullptr, nullptr};
-    unsigned long long launches_per_iteration = 0;
-    static const int use_graph = [] {
-        const char* v = getenv("SPMV_B200_PR_GRAPH");
-        return v ? atoi(v) : 1;
-    }();
-    if (use_graph && config->max_iterations >= 4 && cudaStreamCreate(&gs) == cudaSuccess) {
-        for (int p = 0; p < 2; ++p) {
-            cudaGraph_t g = nullptr;
-            const unsigned long long before = launch_count();
-            bool good = cudaStreamBeginCapture(gs, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
-            if (good) {
-                const int r = enqueue_iteration(p == 0 ? d_a : d_b, p == 0 ? d_b : d_a, p, gs);
-                good = cudaStreamEndCapture(gs, &g) == cudaSuccess && r == 0 && g != nullptr;
-            }
-            launches_per_iteration = launch_count() - before;
-            count_launches(-static_cast<int>(launches_per_iteration));  // captured, not launched
-            if (good) good = cudaGraphInstantiate(&exec[p], g, 0) == cudaSuccess;
-            if (g) cudaGraphDestroy(g);
-            if (!good) {
-                cudaGetLastError();
-                for (int q = 0; q < 2; ++q) {
-                    if (exec[q]) cudaGraphExecDestroy(exec[q]);
-                    exec[q] = nullptr;
-                }
-                break;
-            }
-        }
-    }
-    const bool replay = exec[0] && exec[1];
+    PrIterationGraphs graphs;
+    if (PrIterationGraphs::wanted(config->max_iterations) && cudaStreamCreate(&gs) == cudaSuccess)
+        graphs.capture(gs, [&](int p) { return enqueue_iteration(p ? run.b : run.a, p ? run.a : run.b, p, gs); });
+    const bool replay = graphs.ready();
     cudaStream_t loop_stream = replay ? gs : stream;
     for (int it = 0; it < config->max_iterations; ++it) {
         const int slot = it & 1;
         if (replay) {
-            if (cudaGraphLaunch(exec[slot], gs) != cudaSuccess) {
-                cudaGetLastError();
+            if (!graphs.launch(slot, gs)) {
                 rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
                 break;
             }
-            count_launches(static_cast<int>(launches_per_iteration));
         } else {
             rc = enqueue_iteration(r_old, r_new, slot, stream);
             if (rc != 0) break;  // the reference also leaves the loop on a failed SpMV (:105-107)
@@ -376,23 +364,16 @@ int pagerank_device(const CSRMatrix* adj, const PageRankConfig* config, float* d
     if (pending.valid && rc == 0) conv = settle(pending) && rc == 0;
     cudaEventDestroy(ev[0]);
     cudaEventDestroy(ev[1]);
-    if (gs) cudaStreamSynchronize(gs);  // a speculative iteration may still be running
-    for (int q = 0; q < 2; ++q)
-        if (exec[q]) cudaGraphExecDestroy(exec[q]);
-    if (gs) cudaStreamDestroy(gs);
-    // final vector (:135-139) and normalisation (:142-150)
-    if (normalize) launch_normalize(fin, n, d_ranks, plan->tmp, stream);
-    else cudaMemcpyAsync(d_ranks, fin, sizeof(float) * n, cudaMemcpyDeviceToDevice, stream);
-    cudaError_t e = cudaStreamSynchronize(stream);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        if (rc == 0) rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
+    if (gs) {
+        cudaStreamSynchronize(gs);  // a speculative iteration may still be running
+        cudaStreamDestroy(gs);
     }
+    const int wr = run.write_ranks(fin, n, normalize, d_ranks, stream);
+    if (rc == 0) rc = wr;
     if (iterations) *iterations = iters;
     if (final_residual) *final_residual = residual;
     if (converged) *converged = conv;
     if (l1_residual) *l1_residual = l1;
-    cleanup();
     return rc;
 }
 
@@ -455,9 +436,8 @@ int pagerank_to_host(const CSRMatrix* adj_matrix, const PageRankConfig* config, 
     }
     if (n <= 0) return 0;
 
-    const float init = 1.0f / n;
-    auto fill_initial = [&]() {  // what the reference returns when its first SpMV fails (:105-107, :135-150)
-        for (int i = 0; i < n; ++i) result.ranks[i] = init;
+    // the reference's final normalisation (:142-150): sequential fp32 sum, then every entry divided by it
+    auto normalise_literally = [&]() {
         float sum = 0.0f;
         for (int i = 0; i < n; ++i) sum += result.ranks[i];
         if (sum > 0.0f)
@@ -480,20 +460,17 @@ int pagerank_to_host(const CSRMatrix* adj_matrix, const PageRankConfig* config, 
     const int rc = pagerank_device(adj_matrix, config, d_ranks, &iters, &residual, &conv, nullptr,
                                    !literal_normalisation, nullptr, 0, d_pvec);
     cudaFree(d_pvec);
-    if (rc != 0 && iters == 0) {
+    if (rc != 0 && iters == 0) {  // what the reference returns when its first SpMV fails (:105-107, :135-150)
         cudaFree(d_ranks);
-        fill_initial();
+        const float init = 1.0f / n;
+        for (int i = 0; i < n; ++i) result.ranks[i] = init;
+        normalise_literally();
         return 0;
     }
     cudaError_t e = cudaMemcpy(result.ranks, d_ranks, sizeof(float) * n, cudaMemcpyDeviceToHost);
     cudaFree(d_ranks);
     if (e != cudaSuccess) throw CudaException(e);
-    if (literal_normalisation) {
-        float sum = 0.0f;
-        for (int i = 0; i < n; ++i) sum += result.ranks[i];
-        if (sum > 0.0f)
-            for (int i = 0; i < n; ++i) result.ranks[i] /= sum;
-    }
+    if (literal_normalisation) normalise_literally();
     result.iterations = iters;
     result.final_residual = residual;
     result.converged = conv;

@@ -203,11 +203,6 @@ const NcclApi& nccl() {
     return api;
 }
 
-int env_int(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 }  // namespace
 
 bool nccl_available() { return nccl().ok; }
@@ -237,9 +232,8 @@ struct PrDist {
     HostHistoryEntry* d_hist = nullptr;
     int hist_cap = 0;
     NcclComm nccl_comm = nullptr;
-    cudaGraphExec_t graph[2] = {nullptr, nullptr};
+    PrIterationGraphs graphs;  // kept across runs
     bool dangling_ready = false;
-    unsigned long long launches_per_iteration = 0;
 
     float* vec(int b) const { return symmetric ? static_cast<float*>(r[b].local) : plain_r[b]; }
 };
@@ -248,8 +242,6 @@ namespace {
 
 void free_all(PrDist* d) {
     if (!d) return;
-    for (int q = 0; q < 2; ++q)
-        if (d->graph[q]) cudaGraphExecDestroy(d->graph[q]);
     if (d->nccl_comm && nccl().ok) nccl().CommDestroy(d->nccl_comm);
     if (d->plan) pr_plan_destroy(d->plan);
     if (d->symmetric) {
@@ -386,10 +378,7 @@ int pr_dist_set_personalization(PrDist* d, const float* v_host) {
     // nothing of an earlier run still reads the old slice, and the cached iteration graphs, which hold its
     // address (or none), are dropped: the next run captures them again
     cudaStreamSynchronize(d->stream);
-    for (int q = 0; q < 2; ++q) {
-        if (d->graph[q]) cudaGraphExecDestroy(d->graph[q]);
-        d->graph[q] = nullptr;
-    }
+    d->graphs.reset();
     cudaFree(d->d_pvec);
     d->d_pvec = nullptr;
     int rc = pr_personalization_upload(v_host, d->n, d->row_offset, d->rows, &d->d_pvec, d->stream);
@@ -417,13 +406,8 @@ int setup_dangling(PrDist* d) {
     bool ok = true;
     if (d->world == 1) {
         double* cs = nullptr;
-        ok = cudaMalloc(&cs, sizeof(double) * (n ? n : 1)) == cudaSuccess;
-        if (ok) {
-            cudaMemsetAsync(cs, 0, sizeof(double) * n, d->stream);
-            ok = launch_colsum(A, cs, d->stream) == cudaSuccess &&
-                 launch_dangling_bits(cs, d->n, d->n, d->d_bits, d->stream) == cudaSuccess &&
-                 cudaStreamSynchronize(d->stream) == cudaSuccess;
-        }
+        ok = cudaMalloc(&cs, sizeof(double) * (n ? n : 1)) == cudaSuccess &&
+             pr_dangling_bits(A, cs, d->d_bits, d->stream) == cudaSuccess && cudaStreamSynchronize(d->stream) == cudaSuccess;
         cudaFree(cs);
         return ok ? 0 : -1;
     }
@@ -581,33 +565,11 @@ int pr_dist_run(PrDist* d, const PageRankConfig* config, int fixed_iterations, P
 
     // ---- CUDA graphs of the two ping-pong iterations (fused modes; NCCL calls stay eager) ----------
     const bool fused = d->world == 1 || d->exchange != kExchangeNccl;
-    static const int use_graph = env_int("SPMV_B200_PR_GRAPH", 1);
-    if (fused && use_graph && !d->graph[0] && limit >= 4) {
-        for (int p = 0; p < 2; ++p) {
-            cudaGraph_t g = nullptr;
-            const unsigned long long before = launch_count();
-            bool good = cudaStreamBeginCapture(d->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
-            if (good) {
-                const int r = enqueue_iteration(d, p, config->damping_factor);
-                good = cudaStreamEndCapture(d->stream, &g) == cudaSuccess && r == 0 && g != nullptr;
-            }
-            d->launches_per_iteration = launch_count() - before;
-            count_launches(-static_cast<int>(d->launches_per_iteration));  // captured, not launched
-            if (good) good = cudaGraphInstantiate(&d->graph[p], g, 0) == cudaSuccess;
-            if (g) cudaGraphDestroy(g);
-            if (!good) {
-                cudaGetLastError();
-                for (int q = 0; q < 2; ++q) {
-                    if (d->graph[q]) cudaGraphExecDestroy(d->graph[q]);
-                    d->graph[q] = nullptr;
-                }
-                break;
-            }
-        }
-    }
+    if (fused && !d->graphs.ready() && PrIterationGraphs::wanted(limit))
+        d->graphs.capture(d->stream, [&](int p) { return enqueue_iteration(d, p, config->damping_factor); });
     // every rank replays or none does (a rank that failed to capture would still work, but keep the
     // launch pattern identical everywhere)
-    const bool replay = agree(d->comm, d->graph[0] && d->graph[1]);
+    const bool replay = agree(d->comm, d->graphs.ready());
 
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaEventCreate(&ev0);
@@ -636,12 +598,10 @@ int pr_dist_run(PrDist* d, const PageRankConfig* config, int fixed_iterations, P
     for (int it = 0; it < limit; ++it) {
         const int from = it & 1;
         if (replay) {
-            if (cudaGraphLaunch(d->graph[from], d->stream) != cudaSuccess) {
-                cudaGetLastError();
+            if (!d->graphs.launch(from, d->stream)) {
                 rc = static_cast<int>(SpMVError::KERNEL_LAUNCH);
                 break;
             }
-            count_launches(static_cast<int>(d->launches_per_iteration));
         } else {
             rc = enqueue_iteration(d, from, config->damping_factor);
             if (rc != 0) break;
@@ -686,7 +646,7 @@ int pr_dist_run(PrDist* d, const PageRankConfig* config, int fixed_iterations, P
     out->device_seconds = ms * 1e-3;
     out->wall_seconds = std::chrono::duration<double>(wall1 - wall0).count();
     out->graph_replay = replay ? 1 : 0;
-    out->kernels_per_iteration = static_cast<int>(d->launches_per_iteration);
+    out->kernels_per_iteration = static_cast<int>(d->graphs.launches_per_iteration);
     return rc;
 }
 

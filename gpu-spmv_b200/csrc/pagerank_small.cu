@@ -149,19 +149,14 @@ pagerank_small_kernel(SmallArgs a) {
     }
 }
 
-int small_env(const char* name, int fallback) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
-
 }  // namespace
 
 // Does the one-kernel loop apply?  Small graphs only (measured, profiles/r2_small_pagerank.txt: it wins up to n = 4096,
 // loses from n = 65536 on, where the merge-path step -- balanced over all SMs, hub-column / segmented plans -- takes over).  SPMV_B200_PR_SMALL=0 disables it, =2 forces it.
 bool pagerank_small_applies(int n, int nnz) {
-    static const int mode = small_env("SPMV_B200_PR_SMALL", 1);
-    static const int max_rows = small_env("SPMV_B200_PR_SMALL_ROWS", 8192);
-    static const int max_nnz = small_env("SPMV_B200_PR_SMALL_NNZ", 1 << 18);
+    static const int mode = env_int("SPMV_B200_PR_SMALL", 1);
+    static const int max_rows = env_int("SPMV_B200_PR_SMALL_ROWS", 8192);
+    static const int max_nnz = env_int("SPMV_B200_PR_SMALL_NNZ", 1 << 18);
     if (mode == 0 || n <= 0) return false;
     return mode == 2 || (n <= max_rows && nnz <= max_nnz);
 }
