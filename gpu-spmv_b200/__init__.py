@@ -508,6 +508,50 @@ def pagerank_personalized_batch(A, V, config=None, capacity=0):
     return ranks, it, res, conv, hist
 
 
+# ------------------------------- per-seed top-K personalized PageRank (libspmv_b200_ppr_topk.so) ----
+_ppr_topk = None
+
+
+def ppr_topk_lib():
+    """libspmv_b200_ppr_topk.so, loaded on first use: importing the package does not need it."""
+    global _ppr_topk
+    if _ppr_topk is None:
+        _ppr_topk = capi.load_ppr_topk()
+    return _ppr_topk
+
+
+def pagerank_personalized_batch_top_k(A, V, top, config=None, capacity=0):
+    """The `top` best nodes of each of k personalized PageRank vectors of the graph A (device CSR), without the
+    dense (n, k) rank matrix.
+
+    V as in pagerank_personalized_batch.  Returns (ids, vals, iterations, residual, converged, history): ids (int32)
+    and vals (float32) are (k, top) torch tensors on the current CUDA device; row c holds the min(top, n) largest
+    ranks of vector c, bit for bit those of pagerank_personalized_batch, by rank descending then node id ascending,
+    padded with (-1, 0.0).  The others are as in pagerank_personalized_batch.  Raises RuntimeError with the
+    library's status on a rejected input (top outside [1, 1024] among them)."""
+    import torch
+    lib_t = ppr_topk_lib()
+    n = A.contents.num_rows if A else 0
+    k, offsets, nodes, weights = _teleport_columns(V, n)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    rows = max(int(top), 0)
+    ids = torch.empty((k, rows), dtype=torch.int32, device=dev)
+    vals = torch.empty((k, rows), dtype=torch.float32, device=dev)
+    it = np.zeros(k, np.int32)
+    res = np.zeros(k, np.float32)
+    conv = np.zeros(k, np.bool_)
+    hist = np.full((k, capacity), np.nan, dtype=np.float32)
+    cfg = C.byref(config) if config is not None else None
+    rc = lib_t.spmv_b200_pagerank_personalized_batch_top_k(
+        A, cfg, k, offsets.ctypes.data_as(capi.c_int_p), nodes.ctypes.data_as(capi.c_int_p),
+        weights.ctypes.data_as(capi.c_float_p) if weights is not None else None, int(top), dptr(ids), dptr(vals),
+        it.ctypes.data_as(capi.c_int_p), res.ctypes.data_as(capi.c_float_p), conv.ctypes.data_as(C.POINTER(C.c_bool)),
+        hist.ctypes.data_as(capi.c_float_p) if capacity > 0 else None, capacity)
+    if rc != 0:
+        raise RuntimeError(f"pagerank_personalized_batch_top_k: {spmv_error_string(rc)}")
+    return ids, vals, it, res, conv, hist
+
+
 # --------------------------------------------------------------- benchmark ----
 
 def make_bench_config(num_warmup_runs=5, num_runs=20, compare_cpu=True):

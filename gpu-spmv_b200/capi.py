@@ -231,6 +231,29 @@ def load_ppr(path=PPR_LIB_PATH):
     return lib
 
 
+# ---- include/spmv_b200_ppr_topk.h: libspmv_b200_ppr_topk.so (per-seed top-K personalized PageRank) ----
+PPR_TOPK_LIB_PATH = os.path.join(os.path.dirname(LIB_PATH), "libspmv_b200_ppr_topk.so")
+
+PPR_TOPK_PROTOTYPES = {
+    "spmv_b200_pagerank_personalized_batch_top_k": (C.c_int, [CSR_P, PRC_P, C.c_int, c_int_p, c_int_p, c_float_p, C.c_int,
+                                                              C.c_void_p, C.c_void_p, c_int_p, c_float_p,
+                                                              C.POINTER(C.c_bool), c_float_p, C.c_int]),
+    "spmv_b200_ppr_topk_launch_count": (C.c_ulonglong, []),
+}
+
+
+def load_ppr_topk(path=PPR_TOPK_LIB_PATH):
+    """dlopen libspmv_b200_ppr_topk.so (it loads libspmv_b200.so from its own directory) and attach prototypes."""
+    if not os.path.exists(path):
+        raise ImportError(f"{path} not found: build it with `make -C gpu-spmv_b200/csrc` (there is no CPU fallback)")
+    lib = C.CDLL(path)
+    for name, (restype, argtypes) in PPR_TOPK_PROTOTYPES.items():
+        fn = getattr(lib, name)
+        fn.restype = restype
+        fn.argtypes = argtypes
+    return lib
+
+
 def load(path=LIB_PATH):
     """dlopen the library and attach prototypes.  Raises if it is missing:
     there is deliberately no fallback implementation."""

@@ -167,6 +167,15 @@ __device__ __forceinline__ float pr_row_value(float damping, float y, float ctx,
     return __fadd_rn(__fadd_rn(dy, __fmul_rn(ctx, v)), __fmul_rn(teleport, v));
 }
 
+// ---- ordering ----------------------------------------------------------------
+
+// Order-preserving uint32 image of a float for radix selection: larger float <=> larger key (NaN sorts high);
+// -0 and +0 map to the same key.
+__device__ __forceinline__ unsigned order_key(float v) {
+    const unsigned u = v == 0.0f ? 0u : __float_as_uint(v);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
 // ---- warp reductions ---------------------------------------------------------
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -27,10 +27,7 @@ constexpr int kBlock = 256;
 constexpr int kPerThread = 16;
 constexpr int kChunk = kBlock * kPerThread;  // elements per CTA in the ordered passes
 
-__device__ __forceinline__ unsigned order_key(float v) {  // larger float <=> larger key (NaN sorts high)
-    const unsigned u = v == 0.0f ? 0u : __float_as_uint(v);  // -0 and +0 compare equal
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
+using dev::order_key;
 
 // histogram of byte `shift / 8` of the keys whose higher bytes equal `prefix`
 __global__ void __launch_bounds__(kBlock)
