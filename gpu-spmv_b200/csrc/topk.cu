@@ -9,7 +9,8 @@
 //   2. every element above the threshold is appended to the result (fewer than k);
 //   3. elements EQUAL to the threshold fill the remaining places in ascending id order
 //      (per-chunk counts -> prefix -> ordered write), so the result is deterministic;
-//   4. the k pairs are downloaded and ordered on the host: rank descending, id ascending.
+//   4. the k pairs are downloaded and ordered on the host by the same key: rank descending, id
+//      ascending (a NaN with the sign bit clear above +Inf, one with it set below -Inf; -0 equals +0).
 // "identical top-k up to ties" (north_star): values are exactly those of pagerank_top_k;
 // among equal ranks the reference's order is unspecified (std::partial_sort), ours is by id.
 #include "device_utils.cuh"
@@ -17,6 +18,7 @@
 
 #include <algorithm>
 #include <cub/block/block_scan.cuh>
+#include <cstring>
 #include <vector>
 
 namespace spmv {
@@ -28,6 +30,13 @@ constexpr int kPerThread = 16;
 constexpr int kChunk = kBlock * kPerThread;  // elements per CTA in the ordered passes
 
 using dev::order_key;
+
+// dev::order_key on the host: the same key for the same float
+unsigned host_order_key(float v) {
+    unsigned u = 0;
+    if (v != 0.0f) std::memcpy(&u, &v, sizeof(u));
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
 
 // histogram of byte `shift / 8` of the keys whose higher bytes equal `prefix`
 __global__ void __launch_bounds__(kBlock)
@@ -170,11 +179,16 @@ int pagerank_top_k_device(const float* d_ranks, int n, int k, TopKNode* top_k) {
         cudaStreamSynchronize(stream) != cudaSuccess || cudaGetLastError() != cudaSuccess)
         return fail(SpMVError::KERNEL_LAUNCH);
     cleanup();
+    // by the key the selection used (a strict weak order even with NaNs, which a float comparison is not)
     std::vector<int> order(static_cast<size_t>(kk));
-    for (int i = 0; i < kk; ++i) order[static_cast<size_t>(i)] = i;
+    std::vector<unsigned> keys(static_cast<size_t>(kk));
+    for (int i = 0; i < kk; ++i) {
+        order[static_cast<size_t>(i)] = i;
+        keys[static_cast<size_t>(i)] = host_order_key(vals[static_cast<size_t>(i)]);
+    }
     std::sort(order.begin(), order.end(), [&](int a, int b) {
-        const float va = vals[static_cast<size_t>(a)], vb = vals[static_cast<size_t>(b)];
-        if (va != vb) return va > vb;
+        const unsigned ka = keys[static_cast<size_t>(a)], kb = keys[static_cast<size_t>(b)];
+        if (ka != kb) return ka > kb;
         return ids[static_cast<size_t>(a)] < ids[static_cast<size_t>(b)];
     });
     for (int i = 0; i < kk; ++i) {

@@ -363,7 +363,10 @@ SPMV_B200_API int spmv_b200_partition_rows_weighted(const int* row_ptrs, int num
 /* Top-k of a rank vector that is already in device memory (e.g. spmv_b200_pagerank_device's
  * d_ranks): radix select + ordered tie fill on the device, only min(k, n) pairs are downloaded.
  * Same values as pagerank_top_k (src/pagerank.cu:162-185, which sorts a host copy of all n
- * pairs); equal ranks are ordered by ascending node id (the reference leaves ties unordered). */
+ * pairs); equal ranks are ordered by ascending node id (the reference leaves ties unordered).
+ * The order is that of the fp32 bits read as a sign-magnitude number: -0 and +0 are equal, a NaN
+ * with the sign bit clear ranks above +Inf and one with it set below -Inf, and NaNs are ordered by
+ * their payload (larger payload higher for a positive NaN, lower for a negative one). */
 SPMV_B200_API int spmv_b200_pagerank_top_k_device(const float* d_ranks, int num_nodes, int k,
                                                   spmv_b200_topk_node* top_k);
 

@@ -25,7 +25,8 @@ extern "C" {
  * d_ids, d_vals: device, k * top each, row-major (row c at (size_t)c * top).  Row c holds the min(top, n)
  * largest entries of column c of the batch's d_ranks, with the same fp32 bits, ordered by rank
  * descending, then node id ascending among equal ranks (the order of spmv_b200_pagerank_top_k_device;
- * -0 and +0 are equal); places [n, top) hold id -1 and value 0.0f.
+ * -0 and +0 are equal, a NaN with the sign bit clear ranks above +Inf and one with it set below -Inf);
+ * places [n, top) hold id -1 and value 0.0f.
  *
  * INVALID_ARGUMENT, before any device work: every rejection of the batch (d_ranks aside), top < 1 or
  * top > 1024, d_ids or d_vals NULL.  INVALID_DIMENSION for a non-square adjacency (results zeroed,
