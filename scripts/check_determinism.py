@@ -1,4 +1,4 @@
-"""Runs the sharded PageRank loop several times on one GPU and checks bitwise reproducibility."""
+"""Runs the sharded PageRank loop (one rank) several times on one GPU and checks bitwise reproducibility."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -7,23 +7,22 @@ sp = load_pkg()
 import gpu_spmv_b200.dist as D
 import gpu_spmv_b200.gen as gen
 dev = torch.device("cuda:0")
+torch.cuda.set_device(0)
 scale = int(sys.argv[1]) if len(sys.argv) > 1 else 22
 n, rp, ci, va = gen.rmat_pagerank_csr(scale, 16, 44, dev)
+G = sp.DeviceCSR(n, n, rp, ci, va)
 torch.cuda.synchronize()
-stream = torch.cuda.Stream()
-shard = D.CudaShard(n, 0, rp, ci, va, stream=stream.cuda_stream)
+comm = D.NativeComm(0, 1, f"check-determinism-{os.getpid()}")
+pr = D.NativeShardedPageRank(comm, G, 0, n)
 outs = []
-with torch.cuda.stream(stream):
-    shard.setup_dangling()
+try:
     for rep in range(4):
-        r_a, r_b = torch.empty(n, device=dev), torch.empty(n, device=dev)
-        partial = torch.zeros(3, dtype=torch.float64, device=dev)
-        shard.init_vector(r_a)
-        hist = []
-        fin, it, res, conv, l1 = D.pagerank_loop(shard, r_a, r_b, partial, [0, n], 0.85, 0.0, 0, fixed_iterations=24,
-                                                 on_iteration=lambda i, r: hist.append(r))
-        torch.cuda.synchronize()
-        outs.append(fin.clone())
-        print(rep, "iters", it, "residual", res, "l1", l1, "hist tail", hist[-4:], flush=True)
+        res = pr.run(0.85, 0.0, 24, fixed_iterations=24)
+        outs.append(pr.ranks(dev).clone())
+        print(rep, "iters", res.iterations, "residual", res.final_residual, "l1", res.l1_residual,
+              "exchange", D.EXCHANGE_NAMES.get(res.exchange), "graph replay", res.graph_replay, flush=True)
+finally:
+    pr.close()
+    comm.close()
 for o in outs[1:]:
-    print("bitwise equal to run 0:", bool(torch.equal(o, outs[0])))
+    print("bitwise equal to run 0:", bool(torch.equal(o.view(torch.int32), outs[0].view(torch.int32))))

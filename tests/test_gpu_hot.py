@@ -152,12 +152,13 @@ def test_values_are_read_live_and_plan_follows_uploads(sp, orc, cuda):
     plan.close()
 
 
-def test_pagerank_with_and_without_a_plan(sp, orc, cuda):
-    """The fused PageRank iteration through the planned kernels: same ranks (L1 <= 1e-6 against the
-    f64 restatement of the reference recurrence, src/pagerank.cu:93-150) and the same residuals as
-    through the plain tile kernel.  The whole graph on one GPU takes the segmented stream (different,
-    fixed summation order); a ROW SHARD takes the hub-column kernel, whose r_new slice must equal the
-    plain tile kernel's bit for bit (only the source of x[col] changes)."""
+def test_pagerank_steps_with_and_without_a_plan(sp, orc, cuda):
+    """The fused PageRank iteration through the planned kernels, stepped for a fixed iteration count by a
+    loop written here: same ranks (L1 <= 1e-6 against the f64 restatement of the reference recurrence,
+    src/pagerank.cu:93-150) and the same residuals as through the plain tile kernel.  The whole graph on
+    one GPU takes the segmented stream (different, fixed summation order); a ROW SHARD takes the
+    hub-column kernel, whose r_new slice must equal the plain tile kernel's bit for bit (only the source
+    of x[col] changes)."""
     gen = gen_mod()
     import gpu_spmv_b200.dist as D
     n, rp, ci, va = gen.rmat_pagerank_csr(16, 16, 11, cuda)
@@ -167,8 +168,16 @@ def test_pagerank_with_and_without_a_plan(sp, orc, cuda):
         shard = D.CudaShard(n, 0, rp, ci, va)
         used = shard.set_hot(cap, force=True)
         assert (used == 0) == (cap == 0)
-        out = D.pagerank_sharded(shard, [0, n], 0.85, 0.0, iters, fixed_iterations=iters)
-        outs.append((out.ranks.cpu().numpy(), out.final_residual, out.l1_residual))
+        shard.setup_dangling()
+        r_old, r_new = torch.empty(n, device=cuda), torch.empty(n, device=cuda)
+        partial = torch.zeros(3, dtype=torch.float64, device=cuda)
+        shard.init_vector(r_old)
+        for _ in range(iters):
+            shard(r_old, r_new, partial)
+            shard.dsum.copy_(partial[2:3].to(torch.float32))  # the dangling mass of the vector just written
+            r_old, r_new = r_new, r_old
+        l2, l1 = partial[:2].tolist()
+        outs.append((shard.normalize(r_old).cpu().numpy(), float(np.sqrt(np.float32(l2))), l1))
         shard.close()
     o_ranks, _, o_l2, o_l1, _ = orc.pagerank_f64(n, n, rp.cpu().numpy(), ci.cpu().numpy(), va.cpu().numpy(), 0.85, 0.0,
                                                  iters, fixed_it=iters)
@@ -263,7 +272,7 @@ def test_plan_kind_follows_the_measured_structure(sp, orc, cuda):
     plan2.close()
 
 
-def test_segmented_stream_kernel_forced(cuda):
+def test_whole_file_with_segmented_stream_forced(cuda):
     """The whole file again with SPMV_B200_PLAN=seg (read once per process, hence the subprocess)."""
     if SEG:
         pytest.skip("already forced")

@@ -1,122 +1,51 @@
-"""Sharded PageRank on >= 2 GPUs of one box (one process per GPU, NCCL): the NCCL all-gather
-path, the fused peer-store exchange and the fused NVSwitch-multicast exchange must all reproduce
-the single-GPU result, and must be bitwise identical to each other (same kernels, same summation
-order, only the transport differs).
+"""Sharded PageRank on >= 2 GPUs of one box: the NCCL transport, the fused peer-store exchange and the
+fused NVSwitch-multicast exchange must all reproduce the f64 oracle, and must be bitwise identical to each
+other (same kernels, same summation order, only the transport differs).
 Skipped on boxes with a single GPU."""
 import os
-import socket
 
 import numpy as np
 import pytest
 import torch
-import torch.distributed as dist
-import torch.multiprocessing as mp
 
 pytestmark = pytest.mark.gpu
 
 
-def _free_port():
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    return port
-
-
-def _worker(rank, world, port, scale, out_dir):
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for p in (root, os.path.join(root, "tests")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    from _load_pkg import load_pkg
-    load_pkg()
-    import gpu_spmv_b200.dist as D
-    import gpu_spmv_b200.gen as gen
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    torch.cuda.set_device(rank)
-    dev = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
-    try:
-        n, rp, ci, va = gen.rmat_pagerank_csr(scale, 16, 7, dev)
-        bounds = D.partition_rows(rp, world)
-        srp, sci, sva = D.extract_shard(rp, ci, va, bounds[rank], bounds[rank + 1])
-        torch.cuda.synchronize()
-        results = {}
-        used_multicast = False
-        for mode in ("nccl", "p2p", "multicast"):
-            shard = D.CudaShard(n, bounds[rank], srp, sci, sva)
-            out = D.pagerank_sharded(shard, bounds, 0.85, 1e-6, 100,
-                                     fused_exchange={"nccl": False, "p2p": True, "multicast": "multicast"}[mode])
-            torch.cuda.synchronize()
-            results[mode] = (out.ranks.clone(), out.iterations, out.final_residual, out.converged)
-            if mode == "multicast":
-                used_multicast = bool(shard._multicast)  # False: no NVSwitch multicast here, peer stores were used
-            dist.barrier()
-            shard.disable_peer_exchange()
-            shard.disable_multicast_exchange()
-            shard.close()
-        a, b, c = results["nccl"], results["p2p"], results["multicast"]
-        assert a[1:] == b[1:] == c[1:], (a[1:], b[1:], c[1:])
-        assert torch.equal(a[0], b[0]), "fused peer-store exchange differs from the NCCL all-gather path"
-        assert torch.equal(a[0], c[0]), "multicast exchange differs from the NCCL all-gather path"
-        if rank == 0:
-            print(f"multicast exchange exercised: {used_multicast}")
-        np.save(os.path.join(out_dir, f"ranks_{rank}.npy"), a[0].cpu().numpy())
-        np.save(os.path.join(out_dir, f"meta_{rank}.npy"), np.array([a[1], a[2], float(a[3])]))
-    finally:
-        dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("scale", [14, 18])
-def test_sharded_pagerank_nccl_and_fused_exchange(sp, orc, cuda, tmp_path, scale):
-    world = min(torch.cuda.device_count(), 4)
-    if world < 2:
-        pytest.skip("needs at least 2 GPUs")
-    mp.spawn(_worker, args=(world, _free_port(), scale, str(tmp_path)), nprocs=world, join=True)
-    import gpu_spmv_b200.gen as gen
-    n, rp, ci, va = gen.rmat_pagerank_csr(scale, 16, 7, "cpu")
-    ranks = [np.load(tmp_path / f"ranks_{r}.npy") for r in range(world)]
-    meta = [np.load(tmp_path / f"meta_{r}.npy") for r in range(world)]
-    for r in range(1, world):  # every rank ends with the same full vector
-        assert np.array_equal(ranks[r].view(np.uint32), ranks[0].view(np.uint32)) and np.array_equal(meta[r], meta[0])
-    iters = int(meta[0][0])
-    o_same, _, l2, l1, conv = orc.pagerank_f64(n, n, rp.numpy(), ci.numpy(), va.numpy(), 0.85, 1e-6, 100, fixed_it=iters)
-    assert bool(meta[0][2]) and np.abs(ranks[0].astype(np.float64) - o_same).sum() <= 1e-6
-
-
-# ---- the native path (csrc/pagerank_dist.cu): C++ rendezvous, symmetric buffers, in-kernel barrier ----
-
 def test_native_pagerank_multi_transports_bit_identical(sp, orc, cuda):
     """spmv_b200_pagerank_multi on the GPUs of the box (one process, one host thread per device): multicast,
-    peer stores and NCCL must give bit-identical vectors, within L1 1e-6 of the f64 oracle restatement."""
+    peer stores and NCCL must give bit-identical vectors, within L1 1e-6 of the f64 oracle restatement, for
+    10 fixed iterations and for runs to convergence (tolerance 1e-6, at most 100 iterations), where every
+    transport must also stop at the oracle's iteration."""
     import ctypes as C
     import gpu_spmv_b200.dist as D
     import gpu_spmv_b200.gen as gen
     world = min(torch.cuda.device_count(), 8)
     if world < 2:
         pytest.skip("needs at least 2 GPUs")
-    n, rp, ci, va = gen.rmat_pagerank_csr(18, 16, 7, "cpu")
-    rp_n, ci_n, va_n = rp.numpy(), ci.numpy(), va.numpy()
-    A = sp.csr_from_arrays(n, n, rp_n, ci_n, va_n)
-    iters = 10
-    cfg = sp.make_pagerank_config(0.85, 0.0, iters)
-    o_ranks = orc.pagerank_f64(n, n, rp_n, ci_n, va_n, 0.85, 1e-6, 100, fixed_it=iters)[0]
-    results = {}
-    for name, exchange in (("auto", D.EXCHANGE_AUTO), ("p2p", D.EXCHANGE_P2P), ("nccl", D.EXCHANGE_NCCL)):
-        ranks = np.empty(n, np.float32)
-        res = D.PrDistResult()
-        rc = sp.lib.spmv_b200_pagerank_multi(A, C.byref(cfg), world, None, exchange, 4, iters,
-                                             ranks.ctypes.data_as(C.c_void_p), C.byref(res))
-        assert rc == 0, (name, sp.spmv_error_string(rc))
-        assert res.iterations == iters
-        assert float(np.abs(ranks.astype(np.float64) - o_ranks.astype(np.float64)).sum()) <= 1e-6, name
-        results[name] = (ranks, res.exchange)
-    print("transports used:", {k: D.EXCHANGE_NAMES[v[1]] for k, v in results.items()})
-    assert np.array_equal(results["auto"][0].view(np.uint32), results["p2p"][0].view(np.uint32))
-    assert np.array_equal(results["auto"][0].view(np.uint32), results["nccl"][0].view(np.uint32))
-    sp.csr_destroy(A)
+    for scale, tol, fixed in ((18, 0.0, 10), (14, 1e-6, 0), (18, 1e-6, 0)):
+        n, rp, ci, va = gen.rmat_pagerank_csr(scale, 16, 7, "cpu")
+        rp_n, ci_n, va_n = rp.numpy(), ci.numpy(), va.numpy()
+        A = sp.csr_from_arrays(n, n, rp_n, ci_n, va_n)
+        cfg = sp.make_pagerank_config(0.85, tol, fixed or 100)
+        o_ranks, o_it, _, _, o_conv = orc.pagerank_f64(n, n, rp_n, ci_n, va_n, 0.85, 1e-6, 100, fixed_it=fixed)
+        assert fixed or o_conv
+        results = {}
+        for name, exchange in (("auto", D.EXCHANGE_AUTO), ("p2p", D.EXCHANGE_P2P), ("nccl", D.EXCHANGE_NCCL)):
+            ranks = np.empty(n, np.float32)
+            res = D.PrDistResult()
+            rc = sp.lib.spmv_b200_pagerank_multi(A, C.byref(cfg), world, None, exchange, 4, fixed,
+                                                 ranks.ctypes.data_as(C.c_void_p), C.byref(res))
+            assert rc == 0, (name, sp.spmv_error_string(rc))
+            assert res.iterations == (fixed or o_it), (scale, name, res.iterations, o_it)
+            if not fixed:
+                assert res.converged == 1, (scale, name)
+            assert float(np.abs(ranks.astype(np.float64) - o_ranks.astype(np.float64)).sum()) <= 1e-6, (scale, name)
+            results[name] = (ranks, (res.iterations, res.final_residual, res.converged), res.exchange)
+        print(f"scale {scale}, fixed {fixed}: transports used:", {k: D.EXCHANGE_NAMES[v[2]] for k, v in results.items()})
+        for name in ("p2p", "nccl"):
+            assert results[name][1] == results["auto"][1], (scale, name, results[name][1], results["auto"][1])
+            assert np.array_equal(results["auto"][0].view(np.uint32), results[name][0].view(np.uint32)), (scale, name)
+        sp.csr_destroy(A)
 
 
 def test_plain_c_caller_of_the_multi_gpu_entry_point(cuda):

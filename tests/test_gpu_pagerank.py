@@ -182,6 +182,85 @@ def test_device_resident_api_and_shards_on_one_gpu(sp, orc, cuda):
         s.close()
 
 
+def test_pr_step_p2p_stores_the_shard_into_every_peer_buffer(sp, cuda):
+    """spmv_b200_pr_step_p2p on one GPU, with a two-entry peer table whose other entry is a second buffer on
+    the same device: the shard's rows must land in both buffers bit for bit as spmv_b200_pr_step writes them,
+    with the same partial sums, and no row outside the shard may change.  A row shard through the plain tile
+    kernel and the hub-column kernel, and the whole graph through the segmented stream."""
+    gen = gen_mod()
+    import gpu_spmv_b200.dist as D
+    n, rp, ci, va = gen.rmat_pagerank_csr(14, 16, 5, cuda)
+    shard_rows = (n // 5, (3 * n) // 4)
+    for (lo, hi), cap in ((shard_rows, 0), (shard_rows, 300), ((0, n), -1)):
+        srp, sci, sva = D.extract_shard(rp, ci, va, lo, hi)
+        shard = D.CudaShard(n, lo, srp, sci, sva)
+        assert (shard.set_hot(cap, force=True) == 0) == (cap == 0)
+        shard.setup_dangling()
+        r_old = torch.empty(n, device=cuda)
+        shard.init_vector(r_old)
+        r_old.mul_(gen.vector_pm1(n, 2, cuda).abs() + 0.5)  # not the uniform start vector
+        ref = torch.full((n,), float("nan"), device=cuda)
+        ref_partial = torch.zeros(3, dtype=torch.float64, device=cuda)
+        shard(r_old, ref, ref_partial)
+        torch.cuda.synchronize()
+        for self_rank in (0, 1):
+            mine = torch.full((n,), float("nan"), device=cuda)
+            peer = torch.full((n,), -1.0, device=cuda)
+            table = (C.c_void_p * 2)()
+            table[self_rank], table[1 - self_rank] = mine.data_ptr(), peer.data_ptr()
+            partial = torch.full((3,), float("nan"), dtype=torch.float64, device=cuda)
+            rc = sp.lib.spmv_b200_pr_step_p2p(shard.plan, sp.dptr(r_old), sp.dptr(mine), shard.damping, sp.dptr(shard.dsum),
+                                              sp.dptr(shard.bits), sp.dptr(partial), table, 2, self_rank, None)
+            assert rc == 0, sp.spmv_error_string(rc)
+            torch.cuda.synchronize()
+            for out in (mine, peer):
+                assert torch.equal(out[lo:hi].view(torch.int32), ref[lo:hi].view(torch.int32)), (cap, self_rank)
+            assert torch.equal(partial, ref_partial), (cap, self_rank, partial, ref_partial)
+            assert bool(torch.isnan(mine[:lo]).all()) and bool(torch.isnan(mine[hi:]).all())
+            assert bool((peer[:lo] == -1.0).all()) and bool((peer[hi:] == -1.0).all())
+        shard.close()
+
+
+IPC_CHILD = """
+import ctypes as C, sys
+import torch
+sys.path[:0] = [sys.argv[1], sys.argv[1] + "/tests"]
+from _load_pkg import load_pkg
+sp = load_pkg()
+import gpu_spmv_b200.dist as D
+torch.cuda.set_device(0)
+n = int(sys.argv[3])
+ptr = C.c_void_p()
+rc = sp.lib.spmv_b200_ipc_open(bytes.fromhex(sys.argv[2]), C.byref(ptr))
+assert rc == 0, sp.spmv_error_string(rc)
+got = D._tensor_from_ptr(ptr.value, n, torch.device("cuda:0")).cpu()
+assert torch.equal(got, torch.arange(n, dtype=torch.float32) * 0.5 - 7.0), "the mapped buffer holds other values"
+assert sp.lib.spmv_b200_ipc_close(ptr) == 0
+print("IPC OK", flush=True)
+"""
+
+
+def test_ipc_buffer_mapped_by_a_child_process(sp, cuda):
+    """spmv_b200_ipc_alloc / _open / _close / _free: a child process on the same GPU maps the buffer this process
+    allocated, reads the pattern written here and closes its mapping; then this process frees the buffer."""
+    import subprocess
+    import sys
+    import gpu_spmv_b200.dist as D
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n = 1 << 20
+    ptr, handle = C.c_void_p(), C.create_string_buffer(64)
+    assert sp.lib.spmv_b200_ipc_alloc(n * 4, C.byref(ptr), handle) == 0
+    try:
+        buf = D._tensor_from_ptr(ptr.value, n, cuda)
+        buf.copy_(torch.arange(n, dtype=torch.float32, device=cuda) * 0.5 - 7.0)
+        torch.cuda.synchronize()
+        p = subprocess.run([sys.executable, "-c", IPC_CHILD, root, handle.raw.hex(), str(n)], cwd=root,
+                           stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=300)
+        assert p.returncode == 0 and "IPC OK" in p.stdout, p.stdout[-4000:]
+    finally:
+        assert sp.lib.spmv_b200_ipc_free(ptr) == 0
+
+
 def test_reference_cuda_pagerank_agrees(sp, orc, ref, cuda):
     """Secondary oracle: the reference's own pagerank() (GPU SpMV + host loops) compiled for
     sm_100a from the unmodified sources, where it is trustworthy (n <= 2^15)."""
